@@ -219,6 +219,41 @@ def _(host_ptr, perm, start, count, resident, max_ctas=8):
   return resident.new_empty((count,) + tuple(resident.shape[1:]))
 
 
+# --------------------------------------------------------------------------- K10: frame stacks
+@torch.library.custom_op("derl_b200::gather_frame_stacks", mutates_args=(), device_types="cuda")
+def gather_frame_stacks(frames: Tensor, index: Tensor, perm: Tensor, start: int,
+                        count: int) -> Tensor:
+  """out[j, y, x, c] = frames[index[perm[start + j], c], y, x]: the stacked [count, H, W, k]
+  uint8 minibatch, rebuilt from unique planes (runners/frame_stacks.py).  Plane ids are not
+  checked here; FrameStacks validates caller-supplied ones when it is built."""
+  _dense(frames, "frames", (torch.uint8,))
+  _dense(index, "index", (torch.int32,))
+  _dense(perm, "perm", (torch.int64,))
+  _need(frames.dim() == 3 and frames.shape[0] >= 1, f"frames must be [F, H, W], got "
+        f"{tuple(frames.shape)}")
+  _need(index.dim() == 2 and index.shape[0] >= 1 and index.shape[1] >= 1,
+        f"index must be [S, k], got {tuple(index.shape)}")
+  _need(frames.device == index.device == perm.device, "frames, index and perm must share a device")
+  _need(0 <= start and 0 <= count and start + count <= perm.numel(),
+        f"window [{start}, {start + count}) outside perm of {perm.numel()}")
+  _check_indices(perm, start, count, index.shape[0])
+  n_frames, height, width = frames.shape
+  n_samples, k = index.shape
+  out = frames.new_empty((count, height, width, k))
+  if count == 0:
+    return out
+  with _device_of(frames, "gather_frame_stacks"):
+    _lib.check(_lib.load().derl_b200_gather_frame_stacks(
+        _p(frames), n_frames, height, width, _p(index), n_samples, k, _p(perm), start, count,
+        _p(out), _stream(frames)), "gather_frame_stacks")
+  return out
+
+
+@gather_frame_stacks.register_fake
+def _(frames, index, perm, start, count):
+  return frames.new_empty((count,) + tuple(frames.shape[1:]) + (index.shape[1],))
+
+
 @torch.library.custom_op("derl_b200::gather_columns", mutates_args=(), device_types="cuda")
 def gather_columns(columns: List[Tensor], perm: Tensor, start: int, count: int,
                    moments_col: int = -1) -> List[Tensor]:

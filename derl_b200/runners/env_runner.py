@@ -11,6 +11,8 @@ from abc import ABC, abstractmethod
 import numpy as np
 import torch
 
+from .frame_stacks import FrameStackRollout
+
 _FORWARDED = frozenset(("env", "policy", "horizon", "nsteps", "step_count", "nenvs",
                         "is_exhausted"))
 
@@ -73,10 +75,19 @@ class EnvRunner:
   taken from the forward pass this runner makes on it right after the last step (the same batch
   a GAE bootstrap would evaluate, derl/runners/trajectory_transforms.py:47-50) and kept on the
   device, so `derl_b200.GAE` does not run a second forward or a host round trip for it.
+
+  `pack_frames` (extension, default False): `observations` is yielded as a
+  `runners.frame_stacks.FrameStacks` — every frame plane stored once plus a per-sample stack
+  index, packed on the host one step at a time — instead of stacked arrays: about a quarter of the
+  bytes for 4-frame Atari stacks.  Without `resident_device` the planes are in pinned host memory
+  (TransformInteractions uploads them); with it they are copied to the device step by step.
+  `state["latest_observations"]` stays stacked in both modes.
   """
 
-  def __init__(self, env, policy, horizon, nsteps=None, time_limit=None, resident_device=None):
+  def __init__(self, env, policy, horizon, nsteps=None, time_limit=None, resident_device=None,
+               pack_frames=False):
     self.resident_device = resident_device
+    self.pack_frames = pack_frames
     self.env, self.policy, self.horizon = env, policy, horizon
     self.nsteps = int(nsteps)
     if time_limit is not None and getattr(env.unwrapped, "nenvs", None) is not None:
@@ -109,9 +120,14 @@ class EnvRunner:
           self._resident = _ResidentRollout(self.horizon, self.resident_device)
         resident = self._resident
         resident.begin()
+      frames = FrameStackRollout(self.horizon, self.resident_device) if self.pack_frames else None
 
       def put(key, val, step):
         if resident is not None and key == "next_observations":
+          return
+        if frames is not None and key == "observations":
+          rollout.setdefault(key, None)   # keeps the reference's key order
+          frames.put(step, val)
           return
         if resident is not None and resident.put(key, step, val):
           rollout[key] = resident.buffers[key]
@@ -138,6 +154,8 @@ class EnvRunner:
           self.episode_length = 0
         else:
           obs = next_obs
+      if frames is not None:
+        rollout["observations"] = frames.finish()
       rollout["state"] = dict(latest_observations=obs)
       if resident is not None:
         resident.end()

@@ -17,6 +17,7 @@ import torch
 
 from .. import _lib, ops  # noqa: F401
 from .env_runner import EnvRunner, RunnerWrapper
+from .frame_stacks import FrameStacks
 from .host_column import HostColumn, eligible as _lazy_eligible
 from .row_selection import RowSelection
 from .summary import PeriodicSummaries
@@ -47,6 +48,8 @@ class TransformInteractions(RunnerWrapper):
   def _densify(self, key, val, device):
     if isinstance(val, (torch.Tensor, HostColumn, RowSelection)):
       return val
+    if isinstance(val, FrameStacks):
+      return val.to_device(device)
     try:
       arr = np.asarray(val)
     except ValueError:
@@ -82,11 +85,14 @@ def gather_minibatch(interactions, perm, start, count, host_perm=None, perm_read
   which also reduces the float64 moments of `advantages` (attached as `_derl_moments`).
   fused_gather: a resident `observations` column is handed on as a `RowSelection` (source +
   row indices) for the network's stem kernels to read in place instead of being copied.
+  A `FrameStacks` column is always rebuilt into stacked rows by K10 (fused_gather or not).
   """
   out, narrow = {}, []
   for key, val in interactions.items():
     if key == "state":
       out[key] = val
+    elif isinstance(val, FrameStacks):
+      out[key] = val.gather(perm, start, count)
     elif isinstance(val, HostColumn):
       if fused_gather and key == "observations" and val.complete:
         out[key] = RowSelection(val.resident, perm, start, count)

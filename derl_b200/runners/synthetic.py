@@ -82,6 +82,77 @@ def make_rollout(kind, horizon, nenvs, device="cuda", seed=0, nactions=4, obs_di
   return rollout
 
 
+def make_frame_stack_rollout(horizon, nenvs, device="cuda", seed=0, nactions=4, k=4, height=84,
+                             width=84, reset_prob=0.01, stacked=True):
+  """A seeded atari-shaped rollout whose frame stacks are consistent, in both storage forms.
+
+  Every (env, step) sees one random new frame; a stack holds the env's last k frames, and the
+  first observation after a reset is the baselines-style [f, f, ..., f] (the reset frame
+  repeated).  The rollout starts mid-episode with k-1 frames of history per env, so the planes
+  are (horizon + k - 1) * nenvs.  Returns (stacked_rollout, frames_rollout): the same dict twice,
+  sharing every column but `observations`, which is a stacked uint8 (T, N, H, W, k) array in the
+  first and a `FrameStacks` in the second.  `stacked=False` skips the stacked form (None).
+  `state.latest_observations` is stacked in both.
+  """
+  from .frame_stacks import FrameStacks
+  dev = torch.device(device)
+  gen = torch.Generator(device=dev)
+  gen.manual_seed(seed)
+  lead = (horizon, nenvs)
+  randn = lambda shape: torch.randn(shape, generator=gen, device=dev)
+  rand = lambda shape: torch.rand(shape, generator=gen, device=dev)
+  frames = torch.randint(0, 256, ((horizon + k - 1) * nenvs, height, width), generator=gen,
+                         device=dev, dtype=torch.uint8)
+  latest_frame = torch.randint(0, 256, (nenvs, height, width), generator=gen, device=dev,
+                               dtype=torch.uint8)
+  actions = torch.randint(0, nactions, lead, generator=gen, device=dev, dtype=torch.int64)
+  log_prob = -math.log(nactions) + 0.01 * randn(lead)
+  rdt = torch.float32 if dev.type == "cuda" else torch.float64
+  rewards = (torch.sign(randn(lead)) * (rand(lead) < 0.1)).to(rdt)
+  resets = rand(lead) < reset_prob
+  values = randn(lead + (1,))
+
+  # time of the frame in channel c at step t: max(t - (k-1-c), first step of the episode); the
+  # plane of (env n, time tau) is (tau + k - 1) * nenvs + n
+  done = resets.cpu().numpy()
+  episode_start = np.full(nenvs, -(k - 1), dtype=np.int64)
+  lags = np.arange(k - 1, -1, -1, dtype=np.int64)
+  envs = np.arange(nenvs, dtype=np.int64)
+  index = np.empty(lead + (k,), dtype=np.int32)
+  for t in range(horizon + 1):
+    if t > 0:
+      episode_start = np.where(done[t - 1], t, episode_start)
+    tau = np.maximum(t - lags[None, :], episode_start[:, None])
+    if t < horizon:
+      index[t] = (tau + k - 1) * nenvs + envs[:, None]
+    else:
+      latest_tau = tau
+  # latest stack: planes of steps < horizon from `frames`, the step-`horizon` one is new
+  latest_ids = torch.from_numpy((np.minimum(latest_tau, horizon - 1) + k - 1) * nenvs
+                                + envs[:, None]).to(dev)
+  latest = frames[latest_ids].permute(0, 2, 3, 1).contiguous()
+  fresh = torch.from_numpy(latest_tau == horizon).to(dev)
+  latest = torch.where(fresh[:, None, None, :], latest_frame[..., None], latest)
+
+  index_t = torch.from_numpy(index).to(dev)
+  obs = None
+  if stacked:
+    obs = torch.empty(lead + (height, width, k), dtype=torch.uint8, device=dev)
+    for t in range(horizon):
+      obs[t] = frames[index_t[t].long()].permute(0, 2, 3, 1)
+  columns = dict(actions=actions, log_prob=log_prob, values=values, rewards=rewards,
+                 resets=resets)
+  if dev.type == "cpu":
+    columns = {key: val.numpy() for key, val in columns.items()}
+    latest = latest.numpy()
+    obs = obs.numpy() if obs is not None else None
+  packed = FrameStacks(frames, index_t, validate=False)
+  as_stacked = None if obs is None else dict(observations=obs, **columns,
+                                             state=dict(latest_observations=latest))
+  as_frames = dict(observations=packed, **columns, state=dict(latest_observations=latest))
+  return as_stacked, as_frames
+
+
 class SyntheticRolloutRunner:
   """Yields the same (or freshly seeded) synthetic rollout until `nsteps` env steps."""
 

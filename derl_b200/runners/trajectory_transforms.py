@@ -38,8 +38,9 @@ def to_device(value, device):
 
 
 def _is_array(value):
+  from .frame_stacks import FrameStacks
   from .host_column import HostColumn
-  return isinstance(value, (np.ndarray, torch.Tensor, HostColumn))
+  return isinstance(value, (np.ndarray, torch.Tensor, HostColumn, FrameStacks))
 
 
 class GAE:
@@ -199,7 +200,7 @@ class Take:
     for key, val in trajectory.items():
       if key == "state":
         continue
-      if hasattr(val, "materialize"):   # HostColumn: upload, then index on the device
+      if hasattr(val, "materialize"):   # HostColumn, FrameStacks: stacked on the device, then index
         val = val.materialize()
       if isinstance(val, torch.Tensor):
         axis = self.axis if self.axis >= 0 else self.axis + val.ndim

@@ -30,8 +30,9 @@ extern "C" {
 
 /* 2: derl_b200_stem_conv_relu / derl_b200_stem_backward gained `rows_dev` (fused minibatch gather).
  * 3: derl_b200_ppo_mlp_update (whole PPO update of the MuJoCo-shaped actor-critic in one launch),
- *    derl_b200_stem_conv_relu_mask / derl_b200_stem_backward_masked (tcgen05 stem pair). */
-#define DERL_B200_ABI_VERSION 4
+ *    derl_b200_stem_conv_relu_mask / derl_b200_stem_backward_masked (tcgen05 stem pair).
+ * 5: derl_b200_gather_frame_stacks (minibatch gather out of a frame-plane rollout). */
+#define DERL_B200_ABI_VERSION 5
 
 enum {
   DERL_OK = 0,
@@ -140,6 +141,25 @@ int derl_b200_gather_columns(int n_columns, const void* const* src_dev,
                              const int64_t* perm_dev, int64_t start, int64_t count,
                              int moments_col, double* stats_dev, void* workspace_dev,
                              size_t workspace_bytes, void* stream);
+
+/* ------------------------------------------------------------------ K10: frame-stack gather
+ * The minibatch gather of K2 for a rollout whose `observations` are stored as unique frame
+ * planes (derl_b200/runners/frame_stacks.py): the same two NumPy fancy-index copies of
+ * IterateWithMinibatches (derl/runners/onpolicy.py:44-49, :57-62), now rebuilding each
+ * stacked row from the planes it shares with its neighbours:
+ *     dst[j, y, x, c] = frames[index[perm[start + j] * k + c], y, x]      for j in [0, count)
+ *   frames_dev  uint8 [n_frames, height, width]   unique planes
+ *   index_dev   int32 [n_samples, k]              plane id of every channel of every sample
+ *   dst_dev     uint8 [count, height, width, k]   bit-identical to derl_b200_gather_rows on the
+ *                                                 stacked [n_samples, height, width, k] column
+ * k == 4 with height*width % 16 == 0 and 16-byte aligned frames / index / dst takes the TMA path
+ * (bulk plane copies into shared memory, PRMT interleave, one bulk row store); any other shape a
+ * plain kernel.  Neither checks indices: perm entries must lie in [0, n_samples) and plane ids in
+ * [0, n_frames) (the Python FrameStacks validates caller-supplied ids once, on the host). */
+int derl_b200_gather_frame_stacks(const void* frames_dev, int64_t n_frames, int64_t height,
+                                  int64_t width, const int32_t* index_dev, int64_t n_samples,
+                                  int64_t k, const int64_t* perm_dev, int64_t start, int64_t count,
+                                  void* dst_dev, void* stream);
 
 /* ------------------------------------------------------------------ K3: fused PPO loss
  * Replaces PPOLoss.__call__ (derl/alg/ppo.py:100-108) = policy_loss (:31-64) +
