@@ -8,7 +8,7 @@ import os
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libderl_b200.so")
-ABI_VERSION = 5
+ABI_VERSION = 6
 
 GAE_AUTO, GAE_DIRECT, GAE_TMA = 0, 1, 2
 GAE_STATS = 3
@@ -58,9 +58,6 @@ SIGNATURES = {
                                                _int, _int, _ptr, _size, _ptr]),
     "derl_b200_stem_conv_relu": (_int, [_ptr, _ptr, _i64, _ptr, _ptr, _ptr, _int, _int, _ptr]),
     "derl_b200_space_to_depth": (_int, [_ptr, _i64, _i64, _i64, _i64, _i64, _int, _ptr, _ptr]),
-    "derl_b200_stem_backward_workspace_bytes": (_size, []),
-    "derl_b200_stem_backward": (_int, [_ptr, _ptr, _i64, _ptr, _ptr, _int, _ptr, _ptr, _ptr, _size,
-                                      _ptr]),
     "derl_b200_ppo_mlp_update_smem_bytes": (_size, [_int, _int]),
     "derl_b200_ppo_mlp_update_workspace_bytes": (_size, [_int, _int]),
     "derl_b200_ppo_mlp_update": (_int, [_ptr, _ptr, _ptr, _int, _int, _ptr, _int, _ptr, _ptr, _ptr,
@@ -68,6 +65,7 @@ SIGNATURES = {
                                         _f64, _f64, _f64, _f64, _f64, _f64, _f64, _i64, _ptr, _ptr,
                                         _ptr, _size, _ptr]),
     "derl_b200_stem_conv_relu_mask": (_int, [_ptr, _ptr, _i64, _ptr, _ptr, _ptr, _ptr, _int, _ptr]),
+    "derl_b200_stem_backward_workspace_bytes": (_size, []),
     "derl_b200_stem_backward_masked": (_int, [_ptr, _ptr, _i64, _ptr, _ptr, _int, _ptr, _ptr, _ptr,
                                               _size, _ptr]),
     "derl_b200_gae_host": (_int, [_ptr, _int, _ptr, _ptr, _ptr, _i64, _i64, _f64, _f64, _int,

@@ -1,20 +1,22 @@
 // K7t — backward of the NatureCNN stem (ReLU mask, bias gradient, weight gradient of
-// nn.Conv2d(4, 32, 8, 4) + ReLU, derl/models.py:102-103) on tcgen05.mma kind::i8 with the
-// accumulators in tensor memory.  Same number format as K7 (stem_bwd.cu): the frame operand is the
-// raw uint8 bytes, the masked gradient is quantised per (frame, channel) into two signed 8-bit
-// digit planes (s = max|g| / 127, g ~= s (q1 + q2 / 254)), int32 accumulation per frame is exact,
-// the per-frame tiles are scaled into fp32 running sums.
+// nn.Conv2d(4, 32, 8, 4) + ReLU, derl/models.py:102-103) straight from the uint8 frames, on
+// tcgen05.mma kind::i8 with the accumulators in tensor memory:
+//     g[p, n]     = relu_mask[p, n] ? grad_out[p, n] : 0                      (400 pixels x 32)
+//     dbias[n]   += sum_p g[p, n]
+//     dW[n, c, 4a+i, 4b+j] += (1/255) * sum_{oy,ox} x[4(oy+a)+i, 4(ox+b)+j, c] * g[(oy,ox), n]
+// Number format: the frame operand is the raw uint8 bytes (exact); the masked gradient is
+// quantised per (frame, channel) into two signed 8-bit digit planes (block floating point):
+// s = max_p |g[p, n]| / 127, g ~= s (q1 + q2 / 254), residual <= s / 508.  The int32 accumulation
+// of a frame is exact; the per-frame tiles are scaled into fp32 running sums per CTA, and a second
+// small kernel sums the CTA partials in a fixed order (float64), so the result is deterministic.
 //
-// What the tensor-core formulation removes.  K7 spends its time building mma.sync operands:
-// a byte transpose of the frame into a pixel-fastest layout, ldmatrix / LDS fragment loads, PRMT
-// shifts for the odd kernel columns (589 M warp instructions per 32768 frames, a third of them
-// shared-memory loads).  Here:
+// Operand formulation:
 //   * the frame lands by ONE TMA tensor copy in the row-permuted layout of K6t (plane i = image
 //     rows 4Y + i: for every 4x4-pixel block m' = 21 Y + X its 16 bytes (j, c) at 16 m').  Read
 //     as an MN-MAJOR no-swizzle UMMA operand that is A[tap = 16 i + 4 j + c][k = block m'] — core
 //     matrix = 8 blocks x 16 tap bytes = 128 contiguous bytes, next 8 blocks +128 B (LBO), next
 //     16 taps +7056 B (SBO) — and kernel quadrant (a, b) is the same operand started
-//     16 (21 a + b) bytes later.  No transpose exists any more;
+//     16 (21 a + b) bytes later: no byte transpose, no fragment loads;
 //   * the reduction index is the padded pixel number m = 21 oy + ox (one junk column per output
 //     row, digits 0 there), so the quantiser writes the digits K-major, 16 consecutive m per
 //     16-byte unit: Gq[m / 16][plane * 32 + channel][16] — the canonical K-major operand
@@ -24,7 +26,7 @@
 //     planes of all 32 channels, so the thread that owns it recombines and scales them;
 //   * the ReLU mask arrives as 1 bit per activation (written by K6t with warp ballots, one word
 //     per (32 padded pixels, channel)), not as the fp32 tensor.
-// Per frame HBM reads: 28 224 (frame) + 51 200 (gradient) + 1 792 (mask) = 81 KB (K7: 130.6 KB).
+// Per frame HBM reads: 28 224 (frame) + 51 200 (gradient) + 1 792 (mask) = 81 KB.
 //
 // Roles (576 threads, one persistent CTA per SM): warps 0-15 are workers — quantise frame f+1,
 // then fold frame f's accumulators into their running sums (worker w owns quadrant w / 4 and the
@@ -37,11 +39,6 @@
 #include "tcgen05.cuh"
 
 namespace derl {
-
-// from stem_bwd.cu: fixed-order sum of the per-CTA partials, re-indexed to [32, 4, 8, 8]
-int launch_stem_bwd_reduce(const float* partial_w, const float* partial_b, int ctas,
-                           float* grad_w, float* grad_b, cudaStream_t st);
-
 namespace {
 
 constexpr int kImgBytes = 84 * 84 * 4;
@@ -78,8 +75,11 @@ static_assert(BtSmem::alloc <= 227 * 1024, "shared memory budget");
 // A = frame taps (u8, MN-major), B = gradient digits (s8, K-major), D = int32 [64 x 64]
 constexpr uint32_t kIdesc = umma_idesc_i8(64, 64, /*a u8*/ 0, /*b s8*/ 1, /*a MN-major*/ 1, 0);
 
+// Two-digit quantisation of x in [-127, 127]: q1 = rint(x), q2 = rint((x - q1) * 254) (|q2| <= 127
+// because |x - q1| <= 1/2 exactly).  Rounding by the 1.5 * 2^23 trick keeps the conversion pipe
+// idle; the digits are the low bytes of the biased sums.
 __device__ __forceinline__ void quantise2(float x, unsigned* b1, unsigned* b2) {
-  const float m1 = x + 12582912.f;                    // rint by the 1.5 * 2^23 trick (stem_bwd.cu)
+  const float m1 = x + 12582912.f;
   *b1 = __float_as_uint(m1);
   *b2 = __float_as_uint(__fmaf_rn(x - (m1 - 12582912.f), 254.f, 12582912.f));
 }
@@ -357,6 +357,40 @@ stem_bwd_tc_kernel(const __grid_constant__ CUtensorMap tm_frames, const long lon
   }
 }
 
+// grad_w[n][c][4a+i][4b+j] = (1/255) * sum_cta partial_w[cta][a*2+b][(i*4+j)*4+c][n]
+// Blocks 0 .. kPartial/32 - 1 take 32 consecutive elements of the partial layout (one 128-byte
+// line per CTA partial); the block's 8 warps sum interleaved subsets of the CTAs and the subsets
+// are then added in fixed order.  The last block sums the bias partials the same way.
+__global__ void __launch_bounds__(256)
+stem_bwd_reduce_kernel(const float* __restrict__ partial_w, const float* __restrict__ partial_b,
+                       int ctas, float* __restrict__ grad_w, float* __restrict__ grad_b) {
+  constexpr int kSlots = 8;
+  __shared__ double slot[kSlots][32];
+  const int lane = threadIdx.x & 31, k = threadIdx.x >> 5;
+  const bool bias = blockIdx.x == kPartial / 32;
+  const float* src = bias ? partial_b + lane : partial_w + (size_t)blockIdx.x * 32 + lane;
+  const size_t pitch = bias ? kCh : kPartial;
+  double s = 0.0;
+#pragma unroll 4
+  for (int b = k; b < ctas; b += kSlots) s += (double)__ldg(src + (size_t)b * pitch);
+  slot[k][lane] = s;
+  __syncthreads();
+  if (threadIdx.x < 32) {
+    double total = 0.0;
+#pragma unroll
+    for (int q = 0; q < kSlots; ++q) total += slot[q][lane];
+    if (bias) {
+      grad_b[lane] = (float)total;
+    } else {
+      const int e = blockIdx.x * 32 + lane;   // over [4 quadrants][64 taps][32 ch]
+      const int n = e & 31, tap = (e >> 5) & 63, quadrant = e >> 11;
+      const int c = tap & 3, j = (tap >> 2) & 3, i = tap >> 4;
+      const int kh = 4 * (quadrant >> 1) + i, kw = 4 * (quadrant & 1) + j;
+      grad_w[((n * 4 + c) * 8 + kh) * 8 + kw] = (float)(total * (1.0 / 255.0));
+    }
+  }
+}
+
 struct FramesMapCache {
   const void* base[8];
   long long n[8];
@@ -392,25 +426,53 @@ bool frames_map(CUtensorMap* out, const void* base, long long n) {
 
 }  // namespace
 
-int launch_stem_bwd_tc(const uint8_t* frames, const long long* rows, long long batch,
-                       const float* grad_out, const unsigned* mask, int blocked, float* grad_w,
-                       float* grad_b, void* workspace, cudaStream_t st) {
+bool stem_tc_available();
+}  // namespace derl
+
+using namespace derl;
+
+// one CTA per SM: [grid][kPartial] weight partials, then [grid][kCh] bias partials
+extern "C" size_t derl_b200_stem_backward_workspace_bytes(void) {
+  return (size_t)sm_count() * (kPartial + kCh) * sizeof(float);
+}
+
+extern "C" int derl_b200_stem_backward_masked(const uint8_t* frames, const int64_t* rows_dev,
+                                              int64_t batch, const float* grad_out,
+                                              const uint32_t* relu_mask, int blocked,
+                                              float* grad_weight, float* grad_bias,
+                                              void* workspace, size_t workspace_bytes,
+                                              void* stream) {
+  DERL_REQUIRE(frames && grad_out && relu_mask && grad_weight && grad_bias && workspace &&
+                   batch >= 1, "stem_backward_masked: bad arguments");
+  DERL_REQUIRE(blocked == 0 || blocked == 1, "stem_backward_masked: blocked must be 0 or 1");
+  DERL_REQUIRE((((uintptr_t)frames | (uintptr_t)grad_out | (uintptr_t)relu_mask) & 15) == 0,
+               "stem_backward_masked: inputs must be 16-byte aligned");
+  int rc = require_device();
+  if (rc != DERL_OK) return rc;
+  if (workspace_bytes < derl_b200_stem_backward_workspace_bytes()) {
+    set_error("stem_backward_masked: workspace %zu B too small", workspace_bytes);
+    return DERL_E_WORKSPACE;
+  }
+  DERL_REQUIRE(stem_tc_available(), "stem_backward_masked: cuTensorMapEncodeTiled is unavailable");
+  const long long* rows = reinterpret_cast<const long long*>(rows_dev);
   CUtensorMap tm_frames;
   if (!frames_map(&tm_frames, frames, rows ? (1ll << 30) : batch)) {
-    set_error("stem_backward: cuTensorMapEncodeTiled failed (batch %lld)", batch);
+    set_error("stem_backward: cuTensorMapEncodeTiled failed (batch %lld)", (long long)batch);
     return DERL_E_CUDA;
   }
-  if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(stem_bwd_tc_kernel),
-                                   BtSmem::alloc))
-    return rc;
+  if (int rc_attr = ensure_dynamic_smem(reinterpret_cast<const void*>(stem_bwd_tc_kernel),
+                                        BtSmem::alloc))
+    return rc_attr;
+  cudaStream_t st = as_stream(stream);
   long long grid = sm_count();
   if (grid > batch) grid = batch;
   float* partial_w = reinterpret_cast<float*>(workspace);
   float* partial_b = partial_w + (size_t)grid * kPartial;
   stem_bwd_tc_kernel<<<(unsigned)grid, kThreads, BtSmem::alloc, st>>>(
-      tm_frames, rows, grad_out, mask, partial_w, partial_b, batch, blocked);
+      tm_frames, rows, grad_out, relu_mask, partial_w, partial_b, batch, blocked);
   DERL_LAUNCH_CHECK("stem_bwd_tc_kernel");
-  return launch_stem_bwd_reduce(partial_w, partial_b, (int)grid, grad_w, grad_b, st);
+  stem_bwd_reduce_kernel<<<kPartial / 32 + 1, 256, 0, st>>>(partial_w, partial_b, (int)grid,
+                                                           grad_weight, grad_bias);
+  DERL_LAUNCH_CHECK("stem_bwd_reduce_kernel");
+  return DERL_OK;
 }
-
-}  // namespace derl

@@ -7,11 +7,11 @@ distributional heads: those belong to DQN / SAC, outside the hot path).
 
 The hidden conv / linear layers stay library calls (cuDNN / cuBLAS tensor-core kernels); the
 stem — the one layer that touches the uint8 frames — runs on derl_b200's own INT8 tensor-core
-kernels (K6 forward, K7 backward) whenever a reduced-precision tensor-core path is allowed
-(TF32 or autocast).  B200-specific choices around them: an NHWC uint8 frame stack viewed as
-NCHW *is* a channels_last tensor, so the trunk runs channels_last end to end and the
-reference's NCHW `.contiguous()` transpose copy (models.py:123) never happens; strided convs
-with kernel = 2 x stride run as 2x2/1 convs on space-to-depth tensors.
+kernels (K6t / K6 forward; K7t backward of a float32 forward) whenever a reduced-precision
+tensor-core path is allowed (TF32 or autocast).  B200-specific choices around them: an NHWC uint8
+frame stack viewed as NCHW *is* a channels_last tensor, so the trunk runs channels_last end to end
+and the reference's NCHW `.contiguous()` transpose copy (models.py:123) never happens; strided
+convs with kernel = 2 x stride run as 2x2/1 convs on space-to-depth tensors.
 """
 import numpy as np
 import torch
@@ -76,14 +76,13 @@ class _ConvBiasReLU(torch.autograd.Function):
     ctx.conf = (stride, padding)
     return out
 
-  fused_backward = True  # ReLU mask + bias gradient in one derl_b200 kernel (K5)
-
   @staticmethod
   def backward(ctx, grad_out):
     inputs, weight, out = ctx.saved_tensors
     stride, padding = ctx.conf
     chans = out.shape[1]
-    if (_ConvBiasReLU.fused_backward and chans % 4 == 0 and 256 % (chans // 4) == 0
+    # ReLU mask + bias gradient in one derl_b200 kernel (K5) where its shape rules allow
+    if (chans % 4 == 0 and 256 % (chans // 4) == 0
         and out.is_contiguous(memory_format=torch.channels_last)):
       from . import ops  # noqa: F401
       grad_out = grad_out.contiguous(memory_format=torch.channels_last)
@@ -100,23 +99,21 @@ class _ConvBiasReLU(torch.autograd.Function):
 
 
 class _StemConvReLU(torch.autograd.Function):
-  """The 8x8/4 stem + bias + ReLU straight from uint8 frames (derl_b200 K6) forward, optionally
-  emitting the space-to-depth(2) arrangement the next layer consumes.  Backward: K7 (ReLU mask +
-  bias gradient + weight gradient in one INT8 tensor-core pass over the same uint8 frames) for
-  float32 activations; otherwise (bf16 autocast) K5 (ReLU mask + bias gradient) and the weight
-  gradient of the equivalent space-to-depth conv (K4 re-creates the float frames, cuDNN wgrad),
-  mapped back to [32, 4, 8, 8].  With `rows` both kernels read frames[rows] in place: the
+  """The 8x8/4 stem + bias + ReLU straight from uint8 frames (derl_b200 K6t / K6) forward,
+  optionally emitting the space-to-depth(2) arrangement the next layer consumes.  A float32
+  forward that needs a gradient also emits the ReLU mask as bits (K6t), and the backward is K7t
+  (ReLU mask + bias gradient + weight gradient in one INT8 tensor-core pass over the same uint8
+  frames).  Otherwise (bf16 autocast) the backward is K5 (ReLU mask + bias gradient) and the
+  weight gradient of the equivalent space-to-depth conv (K4 re-creates the float frames, cuDNN
+  wgrad), mapped back to [32, 4, 8, 8].  With `rows` the kernels read frames[rows] in place: the
   minibatch gather fused into the layer (runners/row_selection.py)."""
-
-  tensor_memory = True    # float32 activations: the tcgen05 pair K6t / K7t (ReLU mask as bits)
 
   @staticmethod
   def forward(ctx, frames, weight, bias, dtype, out_block, rows=None):
     """rows: int64 indices — the batch is frames[rows], read in place (fused minibatch gather)."""
     mask = None
     wants_backward = any(ctx.needs_input_grad[1:3])   # no mask for rollouts / no_grad forwards
-    if (_StemConvReLU.tensor_memory and dtype == torch.float32 and _StemConvReLU.fused_backward
-        and wants_backward):
+    if dtype == torch.float32 and wants_backward:
       out, mask = torch.ops.derl_b200.stem_conv_relu_mask(frames, weight.contiguous(), bias,
                                                           out_block, rows)
     else:
@@ -130,8 +127,6 @@ class _StemConvReLU(torch.autograd.Function):
     ctx.weight_dtype, ctx.out_block = weight.dtype, out_block
     return out
 
-  fused_backward = True   # K7 / K7t: mask + bias grad + weight grad in one INT8 tensor-core kernel
-
   @staticmethod
   def backward(ctx, grad_out):
     frames, out, rows = ctx.saved_tensors
@@ -139,10 +134,6 @@ class _StemConvReLU(torch.autograd.Function):
     if ctx.has_mask:
       grad_w, grad_b = torch.ops.derl_b200.stem_backward_masked(frames, grad_out, out,
                                                                 ctx.out_block == 2, rows)
-      return None, grad_w.to(ctx.weight_dtype), grad_b, None, None, None
-    if _StemConvReLU.fused_backward and out.dtype == torch.float32:
-      grad_w, grad_b = torch.ops.derl_b200.stem_backward(frames, grad_out, out,
-                                                         ctx.out_block == 2, rows)
       return None, grad_w.to(ctx.weight_dtype), grad_b, None, None, None
     if rows is not None:   # the library route below wants the batch's frames as one tensor
       frames = torch.ops.derl_b200.gather_rows(frames, rows, 0, rows.numel())

@@ -420,39 +420,6 @@ def _(frames, weight, bias, dtype, out_block=1, rows=None):
   return frames.new_empty(shape, dtype=dtype)
 
 
-@torch.library.custom_op("derl_b200::stem_backward", mutates_args=(), device_types="cuda")
-def stem_backward(frames: Tensor, grad_out: Tensor, out: Tensor, blocked: bool,
-                  rows: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:
-  """(grad_weight [32,4,8,8], grad_bias [32]) of relu(conv2d(frames/255, W, b, stride 4)) given
-  the gradient w.r.t. its output and the saved output: channels-last [B,32,20,20] tensors, or
-  their space-to-depth(2) arrangement [B,128,10,10] when `blocked`."""
-  _dense(frames, "frames", (torch.uint8,))
-  _need(tuple(frames.shape[1:]) == (84, 84, 4), f"frames must be [B,84,84,4], got {tuple(frames.shape)}")
-  batch = _check_rows(frames, rows)
-  _need(batch >= 1, "stem_backward needs at least one frame")
-  want = (batch, 128, 10, 10) if blocked else (batch, 32, 20, 20)
-  for name, t in (("grad_out", grad_out), ("out", out)):
-    _need(t.dtype == torch.float32 and tuple(t.shape) == want
-          and t.is_contiguous(memory_format=torch.channels_last),
-          f"{name} must be a channels_last float32 tensor of shape {want}")
-  grad_w = torch.empty((32, 4, 8, 8), dtype=torch.float32, device=frames.device)
-  grad_b = torch.empty(32, dtype=torch.float32, device=frames.device)
-  lib = _lib.load()
-  ws_bytes = lib.derl_b200_stem_backward_workspace_bytes()
-  ws = torch.empty(ws_bytes, dtype=torch.uint8, device=frames.device)
-  with _device_of(frames, "stem_backward"):
-    _lib.check(lib.derl_b200_stem_backward(
-        _p(frames), _p(rows) if rows is not None else None, batch, _p(grad_out), _p(out),
-        int(blocked), _p(grad_w), _p(grad_b), _p(ws), ws_bytes, _stream(frames)), "stem_backward")
-  return grad_w, grad_b
-
-
-@stem_backward.register_fake
-def _(frames, grad_out, out, blocked, rows=None):
-  return frames.new_empty((32, 4, 8, 8), dtype=torch.float32), \
-      frames.new_empty(32, dtype=torch.float32)
-
-
 @torch.library.custom_op("derl_b200::stem_conv_relu_mask", mutates_args=(), device_types="cuda")
 def stem_conv_relu_mask(frames: Tensor, weight: Tensor, bias: Tensor, out_block: int = 1,
                         rows: Optional[Tensor] = None) -> Tuple[Tensor, Tensor]:

@@ -3,7 +3,7 @@
 The reference's minibatch slice copies every selected observation row out of the rollout
 (`derl/runners/onpolicy.py:57-62`) before the network reads it back (`derl/models.py:79-88,
 117-123`).  With `IterateWithMinibatches(fused_gather=True)` the minibatch's `observations`
-is a `RowSelection` instead: the NatureCNN stem kernels (K6 forward, K7 backward) take the
+is a `RowSelection` instead: the NatureCNN stem kernels (K6t forward, K7t backward) take the
 row indices and pull each 28 224-byte row straight out of the resident rollout (SURVEY §8f
 rank 2), so the minibatch copy — one write and one extra read of every frame — never happens.
 Anything else that touches the object gets the materialised tensor (`materialize()`, any

@@ -31,8 +31,10 @@ extern "C" {
 /* 2: derl_b200_stem_conv_relu / derl_b200_stem_backward gained `rows_dev` (fused minibatch gather).
  * 3: derl_b200_ppo_mlp_update (whole PPO update of the MuJoCo-shaped actor-critic in one launch),
  *    derl_b200_stem_conv_relu_mask / derl_b200_stem_backward_masked (tcgen05 stem pair).
- * 5: derl_b200_gather_frame_stacks (minibatch gather out of a frame-plane rollout). */
-#define DERL_B200_ABI_VERSION 5
+ * 5: derl_b200_gather_frame_stacks (minibatch gather out of a frame-plane rollout).
+ * 6: derl_b200_stem_backward (mma.sync stem backward from the float32 activation) removed:
+ *    derl_b200_stem_backward_masked is the stem backward. */
+#define DERL_B200_ABI_VERSION 6
 
 enum {
   DERL_OK = 0,
@@ -274,25 +276,6 @@ int derl_b200_stem_conv_relu(const uint8_t* frames_dev, const int64_t* rows_dev,
                              const float* weight_dev, const float* bias_dev, void* out_dev,
                              int out_dtype, int out_block, void* stream);
 
-/* ------------------------------------------------------------------ K7: stem backward from uint8 frames
- * Backward of the same layer (ReLU mask, bias gradient and weight gradient of
- * nn.Conv2d(4, 32, 8, 4), derl/models.py:102-103) in one pass over the raw frames, the incoming
- * gradient and the saved activation, on the INT8 tensor cores: the gradient is quantised per
- * (frame, channel) into two signed 8-bit digit planes (block floating point, residual <= 1/508
- * of the channel's largest element in that frame), frames are exact.
- *   frames [batch, 84, 84, 4] uint8; grad_out, out: float32 [batch, 400, 32] tiles of the
- *   activation gradient / activation, pixels in plain (oy*20 + ox) order (blocked = 0) or in the
- *   space-to-depth(2) order K6 emits with out_block = 2 (blocked = 1);
- *   grad_weight [32, 4, 8, 8] float32, grad_bias [32] float32 (overwritten);
- *   rows_dev as in derl_b200_stem_conv_relu (NULL, or the fused gather's row indices).
- *   workspace >= derl_b200_stem_backward_workspace_bytes().  Deterministic. */
-size_t derl_b200_stem_backward_workspace_bytes(void);
-int derl_b200_stem_backward(const uint8_t* frames_dev, const int64_t* rows_dev, int64_t batch,
-                            const float* grad_out_dev, const float* out_dev, int blocked,
-                            float* grad_weight_dev,
-                            float* grad_bias_dev, void* workspace_dev, size_t workspace_bytes,
-                            void* stream);
-
 /* ------------------------------------------------------------------ K5: ReLU backward + bias grad
  * One pass over a channels-last activation gradient [rows, channels] (rows = B*H*W):
  *     grad_pre = out > 0 ? grad_out : 0;   bias_grad[c] = sum over rows of grad_pre[:, c]
@@ -353,17 +336,29 @@ int derl_b200_gae_host(const void* rewards_host, int rewards_f64, const float* v
 /* ------------------------------------------------------------------ K6t / K7t: the stem on tcgen05 + tensor memory
  * derl_b200_stem_conv_relu itself runs the tcgen05 kernel for float32 outputs (the mma.sync
  * kernel remains for bf16 outputs and under DERL_STEM_MMA_SYNC=1; results are bit-identical).
- * The two entry points below are the pair a training step uses: the forward additionally emits
- * the ReLU mask as one bit per activation, and the backward consumes that mask instead of
- * re-reading the float32 activation (51 200 B per frame less HBM traffic).
+ * The entry points below are the pair a training step uses: the forward additionally emits the
+ * ReLU mask as one bit per activation, and the backward consumes that mask instead of re-reading
+ * the float32 activation (51 200 B per frame).
  *   relu_mask [batch, 14, 32] uint32: bit l of word (tile t, channel c) = (activation of channel c
  *     at padded pixel m = 32 t + l is > 0), m = 21 oy + ox (ox = 20 and m >= 420 are padding,
  *     bits 0), whatever out_block / blocked says.
- *   out must be 128-byte aligned (TMA store); everything else as in derl_b200_stem_conv_relu /
- *   derl_b200_stem_backward (derl/models.py:102-103,117-123 forward; its autograd backward). */
+ * Forward: out must be 128-byte aligned (TMA store); everything else as in
+ *   derl_b200_stem_conv_relu (derl/models.py:102-103,117-123).
+ * Backward of the same layer (ReLU mask, bias gradient and weight gradient of
+ * nn.Conv2d(4, 32, 8, 4); its autograd backward) in one pass over the raw frames, the incoming
+ * gradient and the mask, on the INT8 tensor cores: the gradient is quantised per (frame, channel)
+ * into two signed 8-bit digit planes (block floating point, residual <= 1/508 of the channel's
+ * largest element in that frame), frames are exact.
+ *   frames [batch, 84, 84, 4] uint8; grad_out float32 [batch, 400, 32] tiles of the activation
+ *   gradient, pixels in plain (oy*20 + ox) order (blocked = 0) or in the space-to-depth(2) order
+ *   the forward emits with out_block = 2 (blocked = 1); frames, grad_out and relu_mask 16-byte
+ *   aligned; grad_weight [32, 4, 8, 8] float32, grad_bias [32] float32 (overwritten);
+ *   rows_dev as in derl_b200_stem_conv_relu (NULL, or the fused gather's row indices).
+ *   workspace >= derl_b200_stem_backward_workspace_bytes().  Deterministic. */
 int derl_b200_stem_conv_relu_mask(const uint8_t* frames_dev, const int64_t* rows_dev, int64_t batch,
                                   const float* weight_dev, const float* bias_dev, float* out_dev,
                                   uint32_t* relu_mask_dev, int out_block, void* stream);
+size_t derl_b200_stem_backward_workspace_bytes(void);
 int derl_b200_stem_backward_masked(const uint8_t* frames_dev, const int64_t* rows_dev,
                                    int64_t batch, const float* grad_out_dev,
                                    const uint32_t* relu_mask_dev, int blocked,

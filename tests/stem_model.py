@@ -1,9 +1,9 @@
 """NumPy model of the arithmetic of the derl_b200 stem kernels (test infrastructure).
 
-K6 (csrc/stem.cu) and K7 (csrc/stem_bwd.cu) evaluate the reference's first layer
-(derl/models.py:102-103,117-123: `.float()/255` -> nn.Conv2d(4, 32, 8, 4) -> nn.ReLU) and its
-backward on the INT8 tensor cores: one operand (the uint8 frame) is exact, the other (weights
-forward, the masked gradient backward) is expressed as two signed 8-bit digit planes,
+K6 / K6t (csrc/stem.cu, csrc/stem_tc.cu) and K7t (csrc/stem_bwd_tc.cu) evaluate the reference's
+first layer (derl/models.py:102-103,117-123: `.float()/255` -> nn.Conv2d(4, 32, 8, 4) -> nn.ReLU)
+and its backward on the INT8 tensor cores: one operand (the uint8 frame) is exact, the other
+(weights forward, the masked gradient backward) is expressed as two signed 8-bit digit planes,
 value ~= s * (q1 + q2 / 254).  This module restates that number format step by step so that
 its error bounds can be pinned on the CPU against the float64 formulation of the reference.
 """
@@ -48,7 +48,7 @@ def stem_forward(frames, weight, bias):
 
 
 def gradient_digits(masked):
-  """csrc/stem_bwd.cu `quantise`: per (frame, channel) s = max|g| / 127; x = g / s;
+  """csrc/stem_bwd_tc.cu `quantise2`: per (frame, channel) s = max|g| / 127; x = g / s;
   q1 = rint(x) and q2 = rint((x - q1) * 254) by the magic-number trick (the second one through
   one fused multiply-add), |q2| <= 127 because |x - q1| <= 1/2."""
   g = masked.astype(F)                                   # [B,20,20,32]
@@ -63,9 +63,10 @@ def gradient_digits(masked):
 
 
 def stem_backward(frames, grad_out, out):
-  """K7: (grad_weight [32,4,8,8], grad_bias [32]) of the layer given the gradient w.r.t. its
-  output and the saved output (both [B,20,20,32]); per-frame int accumulation is exact, frames
-  are combined in float64 here (the kernel: float32 per CTA, then float64 across CTAs)."""
+  """K7t: (grad_weight [32,4,8,8], grad_bias [32]) of the layer given the gradient w.r.t. its
+  output and the saved output (both [B,20,20,32]; the ReLU mask is out > 0); per-frame int
+  accumulation is exact, frames are combined in float64 here (the kernel: float32 per CTA, then
+  float64 across CTAs)."""
   masked = np.where(out > 0, grad_out, 0).astype(F)
   s, q1, q2 = gradient_digits(masked)
   x = patches(frames)

@@ -12,6 +12,8 @@ import derl_b200 as d
 from derl_b200 import _lib
 from oracle import derl_oracle as O
 
+import stem_model
+
 pytestmark = pytest.mark.gpu
 K = torch.ops.derl_b200
 DEV = "cuda"
@@ -722,7 +724,7 @@ def test_graph_replayed_micro_batched_update_with_fused_gather(golden, tf32):
 #    its first steps, so a 1e-3 relative gradient perturbation (TF32's operand rounding) moves
 #    1.7 M parameters by O(lr) in slightly different directions and the 12-sample minibatch
 #    losses drift by ~1 % — for cuDNN/cuBLAS TF32 alone (custom_stem off) just as for the
-#    default path with K6/K7 (measured side by side: worst step 1.65e-2 vs 1.75e-2).  Bound
+#    default path with K6t/K7t (measured side by side: worst step 1.65e-2 vs 1.75e-2).  Bound
 #    3e-2, and the default path must not drift more than 2x what the TF32 library path does.
 TF32_FIRST_LOSS_RTOL = 5e-4
 TF32_LOSS_RTOL = 3e-2
@@ -749,7 +751,7 @@ def _tf32_update(golden, custom_stem, fused_gather):
 @pytest.mark.parametrize("fused_gather", [False, True])
 def test_benchmarked_configuration_tracks_the_fp32_reference_losses(golden, fused_gather):
   """The configuration bench.py times by default — allow_tf32 on (cuDNN/cuBLAS TF32), the INT8
-  stem kernels K6/K7 on, space-to-depth hidden layers on, micro-batched gradient accumulation
+  stem kernels K6t/K7t on, space-to-depth hidden layers on, micro-batched gradient accumulation
   (ragged chunks: 12-row minibatches in chunks of 5), optionally the fused gather — run on the
   reference's golden rollouts and compared with the losses the reference's float32 CPU classes
   produced (tests/golden/live_update_atari.npz).  This pins the benchmarked arithmetic end to
@@ -757,11 +759,11 @@ def test_benchmarked_configuration_tracks_the_fp32_reference_losses(golden, fuse
   assert d.NatureCNNBase.custom_stem and d.NatureCNNBase.space_to_depth_hidden
   launches = _lib.launch_count()
   rel, dsum = _tf32_update(golden, True, fused_gather)
-  assert _lib.launch_count() - launches >= 8 * 3 * 2, "K6/K7 did not run"
-  lib_rel, lib_dsum = _tf32_update(golden, False, False)   # cuDNN/cuBLAS TF32 only, no K6/K7
+  assert _lib.launch_count() - launches >= 8 * 3 * 2, "K6t/K7t did not run"
+  lib_rel, lib_dsum = _tf32_update(golden, False, False)   # cuDNN/cuBLAS TF32 only, no K6t/K7t
   print(f"\n[tf32 parity] default path (fused_gather={fused_gather}): loss rel dev per step "
         f"{np.array2string(rel, precision=2)}, param-sum dev {dsum:.2e} of sum|p|\n"
-        f"[tf32 parity] TF32 library path (no K6/K7):      loss rel dev per step "
+        f"[tf32 parity] TF32 library path (no K6t/K7t):    loss rel dev per step "
         f"{np.array2string(lib_rel, precision=2)}, param-sum dev {lib_dsum:.2e} of sum|p|")
   assert rel[0] <= TF32_FIRST_LOSS_RTOL, rel
   assert rel.max() <= TF32_LOSS_RTOL, rel
@@ -770,8 +772,8 @@ def test_benchmarked_configuration_tracks_the_fp32_reference_losses(golden, fuse
 
 
 def test_stem_kernels_run_in_the_default_configuration():
-  """Guard for the test above: with allow_tf32 the model routes its first layer through K6
-  (forward) and K7 (backward), and with TF32 off it does not."""
+  """Guard for the test above: with allow_tf32 the model routes its first layer through K6t
+  (forward) and K7t (backward), and with TF32 off it does not."""
   from derl_b200 import ops
   frames = torch.randint(0, 256, (6, 84, 84, 4), dtype=torch.uint8, device=DEV)
   torch.manual_seed(0)
@@ -880,64 +882,22 @@ def test_stem_conv_kernel_vs_float32_convolution(dtype):
   torch.backends.cudnn.allow_tf32 = True
 
 
-@pytest.mark.parametrize("blocked", [False, True])
-def test_stem_backward_kernel_vs_float32_autograd(blocked):
-  """K7: ReLU mask + bias gradient + weight gradient from uint8 frames (INT8 MMA, gradient in
-  two 8-bit digit planes per frame and channel) against float32 autograd of the reference
-  formulation evaluated with the SAME ReLU mask (the mask comes from the forward activation;
-  a reduced-precision forward may flip activations within ~1e-4 of zero, which is checked
-  separately): weight gradient within 2e-4 of its largest entry, bias within 1e-5."""
-  torch.backends.cudnn.allow_tf32 = False
-  gen = torch.Generator(device=DEV).manual_seed(21)
-  weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.05
-  bias = torch.randn(32, device=DEV, generator=gen) * 0.1
-  for batch in (1, 3, 310):
-    frames = torch.randint(0, 256, (batch, 84, 84, 4), device=DEV, dtype=torch.uint8, generator=gen)
-    inputs = frames.permute(0, 3, 1, 2).float() / 255
-    exact = torch.relu(torch.nn.functional.conv2d(inputs, weight, bias, stride=4))
-    out = K.stem_conv_relu(frames, weight, bias, torch.float32, 2 if blocked else 1)
-    plain = (K.space_to_depth(out, 2, True) if blocked else out).permute(0, 3, 1, 2)
-    assert int(((plain > 0) != (exact > 0)).sum()) <= max(2, exact.numel() // 20000)
-    grad = torch.randn(exact.shape, device=DEV, generator=gen) * \
-        torch.rand(batch, 1, 1, 1, device=DEV, generator=gen) * 1e-3
-    masked = grad * (plain > 0)
-    want_w = torch.nn.grad.conv2d_weight(inputs, weight.shape, masked, stride=4)
-    want_b = masked.sum((0, 2, 3))
-    g_nhwc = grad.permute(0, 2, 3, 1).contiguous()
-    if blocked:
-      g_nhwc = K.space_to_depth(g_nhwc, 2, False)
-    args = (frames, g_nhwc.permute(0, 3, 1, 2), out.permute(0, 3, 1, 2), blocked)
-    grad_w, grad_b = K.stem_backward(*args)
-    assert grad_w.shape == (32, 4, 8, 8)
-    err_w = (grad_w - want_w).abs().max() / want_w.abs().max()
-    err_b = (grad_b - want_b).abs().max() / want_b.abs().max()
-    assert err_w < 2e-4 and err_b < 1e-5, (batch, float(err_w), float(err_b))
-    again = K.stem_backward(*args)
-    assert torch.equal(again[0], grad_w) and torch.equal(again[1], grad_b)   # deterministic
-  torch.backends.cudnn.allow_tf32 = True
-
-
-def test_stem_kernels_with_fused_row_gather_are_bit_identical():
-  """K6 / K7 with `rows`: frame i of the batch is source[rows[i]], pulled straight out of the
+def test_stem_forward_kernels_with_fused_row_gather_are_bit_identical():
+  """K6 / K6t with `rows`: frame i of the batch is source[rows[i]], pulled straight out of the
   resident rollout (SURVEY §8f rank 2).  Same bytes in, deterministic kernels: bit-identical to
-  running them on the materialised gather, for both output layouts, with repeated rows."""
+  running them on the materialised gather, for both output layouts, with repeated rows (the
+  backward's `rows` is checked by test_stem_tcgen05_pair_against_its_number_format)."""
   gen = torch.Generator(device=DEV).manual_seed(33)
   weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.05
   bias = torch.randn(32, device=DEV, generator=gen) * 0.1
   source = torch.randint(0, 256, (97, 84, 84, 4), device=DEV, dtype=torch.uint8, generator=gen)
-  for count in (1, 5, 300):   # 300 > 97: rows repeat; > 296 CTAs of K7: second frames per CTA
+  for count in (1, 5, 300):   # 300 > 97: rows repeat; > 296 CTAs of K6: second frames per CTA
     rows = torch.randint(0, 97, (count,), device=DEV, generator=gen)
     dense = source[rows]
     for blk in (1, 2):
       for dtype in (torch.float32, torch.bfloat16):
         assert torch.equal(K.stem_conv_relu(source, weight, bias, dtype, blk, rows),
                            K.stem_conv_relu(dense, weight, bias, dtype, blk))
-      out = K.stem_conv_relu(dense, weight, bias, torch.float32, blk).permute(0, 3, 1, 2)
-      grad = (torch.randn(out.shape, device=DEV, generator=gen) * 1e-3).contiguous(
-          memory_format=torch.channels_last)
-      want = K.stem_backward(dense, grad, out, blk == 2)
-      got = K.stem_backward(source, grad, out, blk == 2, rows)
-      assert torch.equal(got[0], want[0]) and torch.equal(got[1], want[1])
   with pytest.raises(ValueError, match="rows"):
     K.stem_conv_relu(source, weight, bias, torch.float32, 1, rows.int())
 
@@ -1001,7 +961,7 @@ def test_fused_gather_minibatches_and_update_match_the_materialised_pipeline():
   assert torch.equal(finals[0][0], finals[1][0])
   for a, b in zip(finals[0][1], finals[1][1]):
     assert torch.equal(a, b)
-  # strict-fp32 network (no K6/K7): the selection is materialised for the library stem
+  # strict-fp32 network (no K6t/K7t): the selection is materialised for the library stem
   torch.backends.cudnn.allow_tf32 = False
   sel = RowSelection(rollout["observations"].reshape(-1, 84, 84, 4),
                      torch.randperm(nsteps * nenvs, device=DEV), 10, 17)
@@ -1478,27 +1438,33 @@ def _expected_relu_mask(plain_out):
 
 
 @pytest.mark.parametrize("blocked", [False, True])
-def test_stem_tcgen05_pair_mask_and_backward(blocked):
+def test_stem_tcgen05_pair_against_its_number_format(blocked):
   """K6t + K7t (the pair a training step uses): the forward's float32 output is the plain
-  `stem_conv_relu` output bit for bit and its ReLU mask is exactly (output > 0) in the padded
-  pixel-tile layout; the backward (tcgen05, frame as an MN-major operand, gradient digits
-  K-major, accumulators folded per frame from tensor memory) agrees with the mma.sync kernel K7
-  given the same inputs to float32 summation-order noise (1e-6 of the largest entry: both
-  accumulate the same exact per-frame integers) and with float32 autograd under the same mask
-  within K7's own tolerance (2e-4 / 1e-5)."""
+  `stem_conv_relu` output bit for bit, its ReLU signs differ from the float32 convolution's only
+  for the few activations within ~1e-4 of zero, and its ReLU mask is exactly (output > 0) in the
+  padded pixel-tile layout.  The backward (tcgen05, frame as an MN-major operand, gradient digits
+  K-major, accumulators folded per frame from tensor memory) under that mask equals the float64
+  gradients of its number format — the dequantised digits s (q1 + q2 / 254) of
+  tests/stem_model.py — to float32 summation-order noise (1e-6 of the largest entry: the per-frame
+  integer sums are exact), and float32 autograd within the format's tolerance (2e-4 / 1e-5).
+  With the fused gather it is bit-identical to the materialised rows, and it is deterministic."""
   torch.backends.cudnn.allow_tf32 = False
   try:
     gen = torch.Generator(device=DEV).manual_seed(5)
     weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.05
     bias = torch.randn(32, device=DEV, generator=gen) * 0.1
     block = 2 if blocked else 1
-    for batch in (1, 4, 150, 333):
+    for batch in (1, 3, 4, 150, 310, 333):
       frames = torch.randint(0, 256, (batch, 84, 84, 4), device=DEV, dtype=torch.uint8,
                              generator=gen)
       out, mask = K.stem_conv_relu_mask(frames, weight, bias, block, None)
       assert torch.equal(out, K.stem_conv_relu(frames, weight, bias, torch.float32, block, None))
       plain = K.space_to_depth(out, 2, True) if blocked else out
       assert torch.equal(mask.to(torch.int64) & 0xffffffff, _expected_relu_mask(plain))
+      inputs = frames.permute(0, 3, 1, 2).float() / 255
+      exact = torch.relu(torch.nn.functional.conv2d(inputs, weight, bias, stride=4))
+      keep = plain.permute(0, 3, 1, 2) > 0
+      assert int((keep != (exact > 0)).sum()) <= max(2, exact.numel() // 20000)
       grad = torch.randn(batch, 32, 20, 20, device=DEV, generator=gen) * \
           torch.rand(batch, 1, 1, 1, device=DEV, generator=gen) * 1e-3
       g_nhwc = grad.permute(0, 2, 3, 1).contiguous()
@@ -1506,12 +1472,14 @@ def test_stem_tcgen05_pair_mask_and_backward(blocked):
         g_nhwc = K.space_to_depth(g_nhwc, 2, False)
       g_in = g_nhwc.permute(0, 3, 1, 2)
       new_w, new_b = K.stem_backward_masked(frames, g_in, mask, blocked, None)
-      old_w, old_b = K.stem_backward(frames, g_in, out.permute(0, 3, 1, 2), blocked, None)
-      scale_w, scale_b = old_w.abs().max(), old_b.abs().max()
-      assert (new_w - old_w).abs().max() <= 1e-6 * scale_w
-      assert (new_b - old_b).abs().max() <= 1e-6 * scale_b
-      inputs = frames.permute(0, 3, 1, 2).float() / 255
-      masked = grad * (plain.permute(0, 3, 1, 2) > 0)
+      masked = grad * keep
+      s, q1, q2 = stem_model.gradient_digits(masked.permute(0, 2, 3, 1).cpu().numpy())
+      digits = torch.from_numpy(s * (q1 + q2 / 254.0)).to(DEV).permute(0, 3, 1, 2)
+      fmt_w = torch.nn.grad.conv2d_weight(frames.permute(0, 3, 1, 2).double(), weight.shape,
+                                          digits, stride=4) / 255.0
+      fmt_b = masked.double().sum((0, 2, 3))
+      assert (new_w - fmt_w).abs().max() <= 1e-6 * fmt_w.abs().max()
+      assert (new_b - fmt_b).abs().max() <= 1e-6 * fmt_b.abs().max()
       want_w = torch.nn.grad.conv2d_weight(inputs, weight.shape, masked, stride=4)
       want_b = masked.sum((0, 2, 3))
       assert (new_w - want_w).abs().max() < 2e-4 * want_w.abs().max()
@@ -1530,25 +1498,28 @@ def test_stem_tcgen05_pair_mask_and_backward(blocked):
     torch.backends.cudnn.allow_tf32 = True
 
 
-def test_model_routes_float32_stem_through_the_tcgen05_pair():
-  """NatureCNNModel under allow_tf32 uses K6t forward (saving the mask, not the activation) and
-  K7t backward; switching `tensor_memory` off gives the mma.sync pair, and the parameter
-  gradients of the two routes agree to 1e-6 of their scale."""
-  from derl_b200 import models
+def test_model_routes_float32_stem_through_the_tcgen05_pair(monkeypatch):
+  """NatureCNNModel in a float32 training step under allow_tf32 runs its stem forward through K6t
+  (`stem_conv_relu_mask`: the mask is saved, not the activation) and its backward through K7t
+  (`stem_backward_masked`), and the stem's weight and bias gradients are bit for bit what that op
+  returns for the arguments the model passed it."""
+  calls = {"stem_conv_relu_mask": [], "stem_backward_masked": []}
+  for name in calls:
+    def record(*args, _op=getattr(K, name), _calls=calls[name]):
+      _calls.append(args)
+      return _op(*args)
+    monkeypatch.setattr(K, name, record)
   frames = torch.randint(0, 256, (40, 84, 84, 4), dtype=torch.uint8, device=DEV)
-  grads = []
-  for tm in (True, False):
-    models._StemConvReLU.tensor_memory = tm
-    try:
-      torch.manual_seed(0)
-      model = d.NatureCNNModel([4, 1])
-      logits, values = model(frames)
-      (logits.square().sum() + values.sum()).backward()
-      grads.append([p.grad.clone() for p in model.parameters()])
-    finally:
-      models._StemConvReLU.tensor_memory = True
-  for a, b in zip(*grads):
-    assert (a - b).abs().max() <= 1e-6 * max(b.abs().max().item(), 1e-12) + 1e-12
+  torch.manual_seed(0)
+  model = d.NatureCNNModel([4, 1])
+  logits, values = model(frames)
+  (logits.square().sum() + values.sum()).backward()
+  monkeypatch.undo()
+  assert [len(v) for v in calls.values()] == [1, 1], calls
+  grad_w, grad_b = K.stem_backward_masked(*calls["stem_backward_masked"][0])
+  stem = next(m for m in model.modules() if isinstance(m, torch.nn.Conv2d))
+  assert stem.kernel_size == (8, 8)
+  assert torch.equal(stem.weight.grad, grad_w) and torch.equal(stem.bias.grad, grad_b)
 
 
 # ------------------------------------------------------------------------------ K9: linear heads

@@ -1,5 +1,5 @@
 """Hardware check of the tcgen05 stem backward (K7t) and of the ReLU mask K6t emits, against
-float32 autograd (tolerances of tests/test_gpu_parity.py) and the legacy mma.sync kernel K7."""
+float32 autograd (tolerances of tests/test_gpu_parity.py)."""
 import os
 import sys
 import time
@@ -68,21 +68,15 @@ def main():
     gw, gb = torch.autograd.grad(pre, (weight, bias), grad.permute(0, 3, 1, 2) * keep)
     for blocked in (False, True):
       g_in = (s2d2(grad) if blocked else grad).permute(0, 3, 1, 2)
-      o_in = (s2d2(out) if blocked else out).permute(0, 3, 1, 2)
       t0 = time.time()
       nw, nb = K.stem_backward_masked(frames, g_in, mask, blocked, None)
       torch.cuda.synchronize()
-      ow, ob = K.stem_backward(frames, g_in, o_in, blocked, None)
-      torch.cuda.synchronize()
       ew = (nw - gw).abs().max().item() / gw.abs().max().item()
       eb = (nb - gb).abs().max().item() / gb.abs().max().item()
-      ew_old = (ow - gw).abs().max().item() / gw.abs().max().item()
-      dn = (nw - ow).abs().max().item() / gw.abs().max().item()
       good = ew < 2e-4 and eb < 1e-5
       ok = ok and good and mask_ok
-      print(f"batch {batch} blocked {int(blocked)}: mask {mask_ok}  dW err {ew:.2e} (K7 {ew_old:.2e}, "
-            f"K7t-K7 {dn:.2e})  db err {eb:.2e}  {'ok' if good else 'BAD'} ({time.time() - t0:.2f}s)",
-            flush=True)
+      print(f"batch {batch} blocked {int(blocked)}: mask {mask_ok}  dW err {ew:.2e}  db err {eb:.2e}  "
+            f"{'ok' if good else 'BAD'} ({time.time() - t0:.2f}s)", flush=True)
     rows = torch.randint(0, batch, (batch + 3,), device="cuda", generator=gen)
     out_r, mask_r = K.stem_conv_relu_mask(frames, weight.detach(), bias.detach(), 2, rows)
     grad_r = torch.randn(batch + 3, 128, 10, 10, device="cuda", generator=gen).contiguous(
@@ -100,22 +94,16 @@ def main():
   out, mask = K.stem_conv_relu_mask(frames, weight.detach(), bias.detach(), 2, None)
   g_in = torch.randn(nb_, 128, 10, 10, device="cuda", generator=gen).contiguous(
       memory_format=torch.channels_last)
-  o_in = out.permute(0, 3, 1, 2)
-  for name, fn, nbytes in (
-      ("K7t tcgen05 (mask)", lambda: K.stem_backward_masked(frames, g_in, mask, True, None),
-       28224 + 51200 + 1600),
-      ("K7 mma.sync (fp32 act)", lambda: K.stem_backward(frames, g_in, o_in, True, None),
-       28224 + 2 * 51200)):
-    fn()
-    s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    s.record()
-    for _ in range(5):
-      fn()
-    e.record()
-    torch.cuda.synchronize()
-    ms = s.elapsed_time(e) / 5
-    print(f"{name}: {ms:.3f} ms per {nb_} frames, {nb_ * nbytes / ms / 1e6:.0f} GB/s of its own "
-          f"algorithmic bytes", flush=True)
+  K.stem_backward_masked(frames, g_in, mask, True, None)
+  s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+  s.record()
+  for _ in range(5):
+    K.stem_backward_masked(frames, g_in, mask, True, None)
+  e.record()
+  torch.cuda.synchronize()
+  ms = s.elapsed_time(e) / 5
+  print(f"K7t: {ms:.3f} ms per {nb_} frames, {nb_ * (28224 + 51200 + 1600) / ms / 1e6:.0f} GB/s of "
+        f"its own algorithmic bytes", flush=True)
   s, e = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
   s.record()
   for _ in range(5):

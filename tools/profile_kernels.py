@@ -101,8 +101,6 @@ def main():
   timed("stem_backward_masked 32768 (K7t)",
         lambda: K.stem_backward_masked(obs[:32768], gact, relu_mask, True),
         32768 * (28224 + 51200.0 + 1792))
-  timed("stem_backward 32768 blocked (K7, mma.sync)",
-        lambda: K.stem_backward(obs[:32768], gact, act, True), 32768 * (28224 + 2 * 51200.0))
   del act, gact, relu_mask
   frames = obs[:16384]
   for dt, nb in ((torch.float32, 5.0), (torch.bfloat16, 3.0)):

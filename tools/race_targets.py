@@ -1,5 +1,5 @@
 """One small launch of every kernel with an mbarrier / TMA pipeline (K1 TMA scan, K2 row gather,
-K6 / K6t stem forward, K7 / K7t stem backward), for `compute-sanitizer --tool racecheck` (shared-
+K6 / K6t stem forward, K7t stem backward), for `compute-sanitizer --tool racecheck` (shared-
 memory hazards) or `--tool memcheck` / `--tool synccheck`:
 
     compute-sanitizer --tool racecheck python tools/race_targets.py [repeats]
@@ -30,18 +30,17 @@ def main():
     frames = torch.randint(0, 256, (400, 84, 84, 4), dtype=torch.uint8, device="cuda", generator=gen)
     perm = torch.randperm(400, device="cuda", generator=gen)
     K.gather_rows(frames, perm, 3, 390)
-    # K6 / K6t / K7 / K7t
+    # K6 / K6t / K7t
     weight = torch.randn(32, 4, 8, 8, device="cuda", generator=gen) * 0.1
     bias = torch.randn(32, device="cuda", generator=gen) * 0.1
     os.environ["DERL_STEM_MMA_SYNC"] = "1"
-    legacy = K.stem_conv_relu(frames, weight, bias, torch.float32, 2, None)
+    K.stem_conv_relu(frames, weight, bias, torch.float32, 2, None)
     os.environ.pop("DERL_STEM_MMA_SYNC")
     out, mask = K.stem_conv_relu_mask(frames, weight, bias, 2, perm)
     K.stem_conv_relu(frames, weight, bias, torch.float32, 1, None)
     grad = torch.randn(400, 128, 10, 10, device="cuda", generator=gen).contiguous(
         memory_format=torch.channels_last)
     K.stem_backward_masked(frames, grad, mask, True, perm)
-    K.stem_backward(frames, grad, legacy.permute(0, 3, 1, 2), True, None)
   torch.cuda.synchronize()
   print("race targets done")
 
