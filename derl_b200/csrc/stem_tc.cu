@@ -1,8 +1,13 @@
 // K6t — the NatureCNN stem forward (conv 8x8 / 4 over uint8 [84,84,4] frames + bias + ReLU,
-// derl/models.py:102-103,117-123) on the 5th-generation tensor cores: tcgen05.mma kind::i8 with
-// the accumulators in tensor memory.  Same arithmetic as the mma.sync kernel in stem.cu (raw
-// uint8 frame bytes x two signed 8-bit digit planes of the weights, exact int32 accumulation,
-// fp32 recombination), hence bit-identical results; what changes is who moves the operands.
+// derl/models.py:102-103,117-123) straight from the uint8 frames, on the 5th-generation tensor
+// cores: tcgen05.mma kind::i8 with the accumulators in tensor memory.
+// Number format: the frame operand is the raw uint8 bytes (exact, no float conversion); the
+// weights are two signed 8-bit digit planes per output channel n: s = max|W[n]| / 127,
+//   W ~= s (q1 + q2 / 254),  q1 = rint(W / s),  q2 = clamp(rint((W - s q1) * 254 / s), +-127),
+// residual <= s / 508.  Both digit planes accumulate exactly in int32 (|acc| < 2^24); the fp32
+// epilogue is y = relu(float(acc1 * 254 + acc2) * (s / 64770) + bias), every step separately
+// rounded (tests/stem_model.py restates it bit for bit).  bf16 outputs are y rounded to nearest
+// even.
 //
 // Operand formulation.  With the frame cut into 4x4-pixel blocks (space-to-depth(4): block
 // (Y, X) = rows 4Y..4Y+3, columns 4X..4X+3, 64 bytes) the 8x8/4 convolution is a 2x2/1
@@ -20,14 +25,16 @@
 // (4 pixel tiles x 4 quadrants x 2 K-halves; ~1 k tensor cycles) issued by one thread.
 // The 64 accumulator columns of a pixel (32 channels x 2 digit planes) sit in ONE tensor-memory
 // lane, so the epilogue thread that owns the pixel recombines the planes, applies scale, /255,
-// bias and ReLU and holds the pixel's 128 output bytes — written to a 128B-swizzled staging tile
-// (conflict-free) that a TMA tensor store drains as two 25.6 KB boxes per frame.
+// bias and ReLU and holds the pixel's 32 outputs — 128 bytes of fp32 written to a 128B-swizzled
+// staging tile, or 64 bytes of bf16 to a 64B-swizzled one (16-byte stores, conflict-free) — that a
+// TMA tensor store drains as two 200-pixel boxes per frame.
 //
 // Roles (576 threads, one persistent CTA per SM): warp 0 = TMA producer (frames, three
 // buffers: HBM latency is ~a frame period, so loads run two frames ahead), warp 1 = MMA issuer + TMEM owner, warps 2-9 / 10-17 = two epilogue groups taking
 // alternate frames (each owns one 256-column accumulator buffer and one staging tile), so that
 // frame f+1's loads and MMAs and frame f's epilogue and frame f-1's store overlap.
 #include <cuda.h>
+#include <cuda_bf16.h>
 
 #include "common.cuh"
 #include "tcgen05.cuh"
@@ -41,7 +48,7 @@ constexpr int kFrameBuf = 29824;              // frame + over-read slack of the 
 constexpr int kOutC = 32, kPixPad = 420;      // padded pixel index m = 21 oy + ox, ox = 20 is junk
 constexpr int kMTiles = 4;                    // 4 x 128 rows
 constexpr int kWBytes = 16 * 64 * 16;         // [k16][n'][16 B]
-constexpr int kStageBytes = 400 * 128;        // one frame's fp32 activation
+constexpr int kStageBytes = 400 * 128;        // one frame's fp32 activation (bf16 uses half)
 constexpr int kEpiWarps = 8;                  // warps per epilogue group: 4 lane quarters x 2 tile parities
 constexpr int kThreads = (2 + 2 * kEpiWarps) * 32;   // 576
 constexpr int kStages = 3;                    // frame buffers: loads run two frames ahead of the MMAs
@@ -64,7 +71,13 @@ static_assert(TcSmem::alloc <= 227 * 1024, "shared memory budget");
 
 constexpr uint32_t kIdesc = umma_idesc_i8(128, 64, /*a u8*/ 0, /*b s8*/ 1, 0, 0);
 
-template <bool kMask>   // kMask: also emit the ReLU mask words (K7t's input)
+__device__ __forceinline__ unsigned pack_bf16(float lo, float hi) {   // round to nearest even
+  const __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
+  return *reinterpret_cast<const unsigned*>(&v);
+}
+
+// kMask: also emit the ReLU mask words (K7t's input).  OT: float or __nv_bfloat16 output.
+template <bool kMask, typename OT>
 __global__ void __launch_bounds__(kThreads, 1)
 stem_conv_relu_tc_kernel(const __grid_constant__ CUtensorMap tm_frames,
                          const __grid_constant__ CUtensorMap tm_out,
@@ -201,6 +214,7 @@ stem_conv_relu_tc_kernel(const __grid_constant__ CUtensorMap tm_frames,
     const int tp = (e % kEpiWarps) >> 2;                // tile parity
     const int gt = tid - (2 + kEpiWarps * g) * 32;      // thread index inside the group
     uint8_t* stage = smem + TcSmem::stage + g * kStageBytes;
+    constexpr int kRow = 32 * sizeof(OT);               // staging bytes per pixel: 128 or 64
     int it = 0, mine = 0;
     for (long long f = first; f < batch; f += stride, ++it) {
       if ((it & 1) != g) continue;
@@ -219,8 +233,10 @@ stem_conv_relu_tc_kernel(const __grid_constant__ CUtensorMap tm_frames,
         int row = oy * 20 + ox;
         if (out_block == 2) row = (((oy >> 1) * 10 + (ox >> 1)) << 2) + ((oy & 1) << 1) + (ox & 1);
         unsigned bits = 0u;       // lane c ends up with channel c's bits of this warp's 32 pixels
-        uint8_t* dst = stage + row * 128;
-        const int sw = row & 7;
+        uint8_t* dst = stage + row * kRow;
+        // TMA swizzle of 16-byte chunks: 128B rows -> chunk ^ (row & 7), 64B -> chunk ^ (row/2 & 3)
+        const int sw = kRow == 128 ? row & 7 : (row >> 1) & 3;
+        unsigned packed[4];       // bf16: the current 8-channel chunk
 #pragma unroll
         for (int half = 0; half < 2; ++half) {   // 16 channels at a time: 32 live accumulator words
           uint32_t v1[16], v2[16];
@@ -247,9 +263,18 @@ stem_conv_relu_tc_kernel(const __grid_constant__ CUtensorMap tm_frames,
               }
               y[k] = x;
             }
-            if (valid) {
-              *reinterpret_cast<float4*>(dst + (((4 * half + c4) ^ sw) << 4)) =
-                  make_float4(y[0], y[1], y[2], y[3]);
+            if constexpr (kRow == 128) {
+              if (valid) {
+                *reinterpret_cast<float4*>(dst + (((4 * half + c4) ^ sw) << 4)) =
+                    make_float4(y[0], y[1], y[2], y[3]);
+              }
+            } else {
+              packed[2 * (c4 & 1)] = pack_bf16(y[0], y[1]);
+              packed[2 * (c4 & 1) + 1] = pack_bf16(y[2], y[3]);
+              if (valid && (c4 & 1)) {
+                *reinterpret_cast<uint4*>(dst + (((2 * half + (c4 >> 1)) ^ sw) << 4)) =
+                    make_uint4(packed[0], packed[1], packed[2], packed[3]);
+              }
             }
           }
         }
@@ -264,7 +289,7 @@ stem_conv_relu_tc_kernel(const __grid_constant__ CUtensorMap tm_frames,
       named_bar_sync(1 + g, kEpiWarps * 32);
       if (gt == 0) {
         tma_store_2d(&tm_out, stage, 0, (int)(f * 400));
-        tma_store_2d(&tm_out, stage + 200 * 128, 0, (int)(f * 400 + 200));
+        tma_store_2d(&tm_out, stage + 200 * kRow, 0, (int)(f * 400 + 200));
         bulk_commit();
       }
       ++mine;
@@ -280,6 +305,7 @@ stem_conv_relu_tc_kernel(const __grid_constant__ CUtensorMap tm_frames,
 }
 
 // ------------------------------------------------------------------ tensor maps (memoised per thread)
+enum MapKind { kFramesMap, kOutF32Map, kOutBf16Map };
 struct MapKey {
   const void* base;
   long long n;
@@ -323,37 +349,38 @@ bool make_frames_map(CUtensorMap* map, const MapKey& key) {
              CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-// out [n * 400 rows][32 f32]; box = 200 rows, 128B swizzle (the staging tile's layout).
+// out [n * 400 rows][32 channels] of fp32 (128 B rows, 128B swizzle) or bf16 (64 B rows, 64B
+// swizzle); box = 200 rows (the staging tile's layout).
 bool make_out_map(CUtensorMap* map, const MapKey& key) {
   TmapEncodeFn enc = tmap_encode_fn();
   if (enc == nullptr) return false;
+  const bool bf16 = key.kind == kOutBf16Map;
   cuuint64_t dims[2] = {32, (cuuint64_t)key.n * 400};
-  cuuint64_t strides[1] = {128};
+  cuuint64_t strides[1] = {bf16 ? 64u : 128u};
   cuuint32_t box[2] = {32, 200};
   cuuint32_t estr[2] = {1, 1};
-  return enc(map, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, const_cast<void*>(key.base), dims, strides,
-             box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
+  return enc(map, bf16 ? CU_TENSOR_MAP_DATA_TYPE_BFLOAT16 : CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2,
+             const_cast<void*>(key.base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+             bf16 ? CU_TENSOR_MAP_SWIZZLE_64B : CU_TENSOR_MAP_SWIZZLE_128B,
              CU_TENSOR_MAP_L2_PROMOTION_NONE, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-}  // namespace
-
-bool stem_tc_available() { return tmap_encode_fn() != nullptr; }
-
-// frames_total: rows of the frames array (>= batch; the gather source when rows != NULL, where
-// the caller may not know it: pass 0 and the map is built for 2^30 frames — the indices are
-// trusted, as in every gather of this library).
+// With rows the frames array is the gather source, whose length the caller may not know: the map
+// is built for 2^30 frames (the indices are trusted, as in every gather of this library).
 int launch_stem_tc(const uint8_t* frames, const long long* rows, long long batch,
-                   long long frames_total, const float* weight, const float* bias, float* out,
+                   const float* weight, const float* bias, void* out, int out_dtype,
                    unsigned* mask_out, int out_block, cudaStream_t st) {
-  if (frames_total <= 0) frames_total = rows ? (1ll << 30) : batch;
+  const bool bf16 = out_dtype == DERL_DTYPE_BF16;
   CUtensorMap tm_frames, tm_out;
-  if (!cached_map(&tm_frames, MapKey{frames, frames_total, 0}, make_frames_map) ||
-      !cached_map(&tm_out, MapKey{out, batch, 1}, make_out_map)) {
+  if (!cached_map(&tm_frames, MapKey{frames, rows ? (1ll << 30) : batch, kFramesMap},
+                  make_frames_map) ||
+      !cached_map(&tm_out, MapKey{out, batch, bf16 ? kOutBf16Map : kOutF32Map}, make_out_map)) {
     set_error("stem_conv_relu: cuTensorMapEncodeTiled failed (batch %lld)", batch);
     return DERL_E_CUDA;
   }
-  auto kern = mask_out != nullptr ? stem_conv_relu_tc_kernel<true> : stem_conv_relu_tc_kernel<false>;
+  auto kern = bf16                ? stem_conv_relu_tc_kernel<false, __nv_bfloat16>
+              : mask_out != nullptr ? stem_conv_relu_tc_kernel<true, float>
+                                    : stem_conv_relu_tc_kernel<false, float>;
   if (int rc = ensure_dynamic_smem(reinterpret_cast<const void*>(kern), TcSmem::alloc)) return rc;
   long long grid = sm_count();
   if (grid > batch) grid = batch;
@@ -363,4 +390,47 @@ int launch_stem_tc(const uint8_t* frames, const long long* rows, long long batch
   return DERL_OK;
 }
 
+}  // namespace
+
+bool stem_tc_available() { return tmap_encode_fn() != nullptr; }
+
 }  // namespace derl
+
+using namespace derl;
+
+extern "C" int derl_b200_stem_conv_relu(const uint8_t* frames, const int64_t* rows, int64_t batch,
+                                        const float* weight, const float* bias, void* out,
+                                        int out_dtype, int out_block, void* stream) {
+  DERL_REQUIRE(out_block == 1 || out_block == 2, "stem_conv_relu: out_block must be 1 or 2");
+  DERL_REQUIRE(frames && weight && bias && out && batch >= 0, "stem_conv_relu: bad arguments");
+  DERL_REQUIRE(out_dtype == DERL_DTYPE_F32 || out_dtype == DERL_DTYPE_BF16,
+               "stem_conv_relu: out_dtype must be DERL_DTYPE_F32 or DERL_DTYPE_BF16");
+  DERL_REQUIRE(((uintptr_t)frames & 15) == 0 && ((uintptr_t)out & 15) == 0,
+               "stem_conv_relu: frames and out must be 16-byte aligned");
+  DERL_REQUIRE(batch * 400 < (1ll << 31), "stem_conv_relu: batch too large");
+  int rc = require_device();
+  if (rc != DERL_OK) return rc;
+  if (batch == 0) return DERL_OK;
+  DERL_REQUIRE(stem_tc_available(), "stem_conv_relu: cuTensorMapEncodeTiled is unavailable");
+  return launch_stem_tc(frames, reinterpret_cast<const long long*>(rows), batch, weight, bias, out,
+                        out_dtype, nullptr, out_block, as_stream(stream));
+}
+
+extern "C" int derl_b200_stem_conv_relu_mask(const uint8_t* frames, const int64_t* rows,
+                                             int64_t batch, const float* weight, const float* bias,
+                                             float* out, uint32_t* relu_mask, int out_block,
+                                             void* stream) {
+  DERL_REQUIRE(out_block == 1 || out_block == 2, "stem_conv_relu_mask: out_block must be 1 or 2");
+  DERL_REQUIRE(frames && weight && bias && out && relu_mask && batch >= 0,
+               "stem_conv_relu_mask: bad arguments");
+  DERL_REQUIRE(((uintptr_t)frames & 15) == 0 && ((uintptr_t)out & 127) == 0 &&
+                   ((uintptr_t)relu_mask & 15) == 0,
+               "stem_conv_relu_mask: frames / mask must be 16-byte, out 128-byte aligned");
+  DERL_REQUIRE(batch * 400 < (1ll << 31), "stem_conv_relu_mask: batch too large");
+  int rc = require_device();
+  if (rc != DERL_OK) return rc;
+  if (batch == 0) return DERL_OK;
+  DERL_REQUIRE(stem_tc_available(), "stem_conv_relu_mask: cuTensorMapEncodeTiled is unavailable");
+  return launch_stem_tc(frames, reinterpret_cast<const long long*>(rows), batch, weight, bias, out,
+                        DERL_DTYPE_F32, relu_mask, out_block, as_stream(stream));
+}

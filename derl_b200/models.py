@@ -7,7 +7,7 @@ distributional heads: those belong to DQN / SAC, outside the hot path).
 
 The hidden conv / linear layers stay library calls (cuDNN / cuBLAS tensor-core kernels); the
 stem — the one layer that touches the uint8 frames — runs on derl_b200's own INT8 tensor-core
-kernels (K6t / K6 forward; K7t backward of a float32 forward) whenever a reduced-precision
+kernels (K6t forward; K7t backward of a float32 forward) whenever a reduced-precision
 tensor-core path is allowed (TF32 or autocast).  B200-specific choices around them: an NHWC uint8
 frame stack viewed as NCHW *is* a channels_last tensor, so the trunk runs channels_last end to end
 and the reference's NCHW `.contiguous()` transpose copy (models.py:123) never happens; strided
@@ -99,7 +99,7 @@ class _ConvBiasReLU(torch.autograd.Function):
 
 
 class _StemConvReLU(torch.autograd.Function):
-  """The 8x8/4 stem + bias + ReLU straight from uint8 frames (derl_b200 K6t / K6) forward,
+  """The 8x8/4 stem + bias + ReLU straight from uint8 frames (derl_b200 K6t) forward,
   optionally emitting the space-to-depth(2) arrangement the next layer consumes.  A float32
   forward that needs a gradient also emits the ReLU mask as bits (K6t), and the backward is K7t
   (ReLU mask + bias gradient + weight gradient in one INT8 tensor-core pass over the same uint8
@@ -174,7 +174,7 @@ class NatureCNNBase(nn.Sequential):
     self.add_module("flatten", nn.Flatten())
     self.add_module("linear", nn.Linear(height * width * convs[-1].out_channels, 512))
 
-  custom_stem = True             # K6: stem conv straight from uint8 frames (needs TF32 allowed
+  custom_stem = True             # K6t: stem conv straight from uint8 frames (needs TF32 allowed
                                  # or autocast: it is a reduced-precision tensor-core path)
   space_to_depth = True          # class-wide switches (tests compare the formulations)
   space_to_depth_hidden = True   # ... also for strided convs after the stem (the 4x4/2 layer):

@@ -374,13 +374,14 @@ def _s2d_backward(ctx, grad):
 space_to_depth.register_autograd(_s2d_backward, setup_context=_s2d_setup)
 
 
-# --------------------------------------------------------------------------- K6: stem conv
+# --------------------------------------------------------------------------- K6t: stem conv
 @torch.library.custom_op("derl_b200::stem_conv_relu", mutates_args=(), device_types="cuda")
 def stem_conv_relu(frames: Tensor, weight: Tensor, bias: Tensor, dtype: torch.dtype,
                    out_block: int = 1, rows: Optional[Tensor] = None) -> Tensor:
   """relu(conv2d(frames/255, weight, bias, stride 4)) for uint8 NHWC frames [B,84,84,4] and the
-  Atari stem weight [32,4,8,8]; returns the channels-last activation [B,20,20,32], or its
-  space-to-depth(2) arrangement [B,10,10,128] when out_block == 2.  `rows` (int64 [B']): the
+  Atari stem weight [32,4,8,8] (K6t); returns the channels-last activation [B,20,20,32], or its
+  space-to-depth(2) arrangement [B,10,10,128] when out_block == 2.  A bfloat16 output is the
+  float32 one rounded to nearest even.  `rows` (int64 [B']): the
   batch is frames[rows] — the minibatch gather fused into the layer, nothing materialised."""
   _dense(frames, "frames", (torch.uint8,))
   batch = _check_rows(frames, rows)

@@ -32,7 +32,7 @@ extern "C" {
  * 3: derl_b200_ppo_mlp_update (whole PPO update of the MuJoCo-shaped actor-critic in one launch),
  *    derl_b200_stem_conv_relu_mask / derl_b200_stem_backward_masked (tcgen05 stem pair).
  * 5: derl_b200_gather_frame_stacks (minibatch gather out of a frame-plane rollout).
- * 6: derl_b200_stem_backward (mma.sync stem backward from the float32 activation) removed:
+ * 6: derl_b200_stem_backward (the stem backward from the float32 activation) removed:
  *    derl_b200_stem_backward_masked is the stem backward. */
 #define DERL_B200_ABI_VERSION 6
 
@@ -254,23 +254,26 @@ int derl_b200_space_to_depth(const void* src_dev, int64_t batch, int64_t height,
                              int64_t channel_bytes, int64_t block, int inverse, void* dst_dev,
                              void* stream);
 
-/* ------------------------------------------------------------------ K6: stem conv on uint8 frames
+/* ------------------------------------------------------------------ K6t: stem conv on uint8 frames
  * The reference's first layer (derl/models.py:102-103,117-123): permute, `.float()/255`,
  * nn.Conv2d(4, 32, 8, 4), nn.ReLU — evaluated straight from the uint8 frames on the INT8
- * tensor cores of sm_100a (raw frame bytes x two signed 8-bit digit planes of the weights,
- * exact int32 accumulation, fp32 recombination), without materialising a floating-point copy
- * of the frames.  Fixed to the Atari stem geometry:
+ * tensor cores of sm_100a (tcgen05.mma with the accumulators in tensor memory: raw frame bytes x
+ * two signed 8-bit digit planes of the weights, exact int32 accumulation, fp32 recombination),
+ * without materialising a floating-point copy of the frames.  One kernel writes float32 or bf16;
+ * the bf16 output is the float32 one rounded to nearest even.  Fixed to the Atari stem geometry:
  *   frames [batch, 84, 84, 4] uint8 NHWC; weight [32, 4, 8, 8] float32 (conv layout); bias [32];
  *   out_block 1: out [batch, 20, 20, 32] channels-last;
  *   out_block 2: out [batch, 10, 10, 128], the space-to-depth(2) arrangement of the same
  *                activation (what derl_b200_space_to_depth would produce from it);
- *   out_dtype DERL_DTYPE_F32 or DERL_DTYPE_BF16;
+ *   out_dtype DERL_DTYPE_F32 or DERL_DTYPE_BF16; frames and out 16-byte aligned;
+ *   batch * 400 < 2^31;
  *   rows_dev  NULL, or `batch` int64 row indices into frames_dev: frame i of the batch is
  *             frames_dev[rows_dev[i]].  This fuses the minibatch gather of
  *             IterateWithMinibatches (derl/runners/onpolicy.py:44-49,57-62) into the layer
  *             (SURVEY §8f rank 2): the kernel pulls each 28 224-byte row straight out of the
  *             resident rollout and the minibatch's observations are never materialised.
  *             Indices are trusted (validate the permutation once, when it is uploaded).
+ * Needs cuTensorMapEncodeTiled from the driver (DERL_E_INVALID without it).
  */
 int derl_b200_stem_conv_relu(const uint8_t* frames_dev, const int64_t* rows_dev, int64_t batch,
                              const float* weight_dev, const float* bias_dev, void* out_dev,
@@ -333,9 +336,7 @@ int derl_b200_gae_host(const void* rewards_host, int rewards_f64, const float* v
                        int64_t N, double gamma, double lambda, int normalize, double epsilon,
                        float* advantages_host, float* value_targets_host, void* stream);
 
-/* ------------------------------------------------------------------ K6t / K7t: the stem on tcgen05 + tensor memory
- * derl_b200_stem_conv_relu itself runs the tcgen05 kernel for float32 outputs (the mma.sync
- * kernel remains for bf16 outputs and under DERL_STEM_MMA_SYNC=1; results are bit-identical).
+/* ------------------------------------------------------------------ K6t / K7t: the stem pair of a training step
  * The entry points below are the pair a training step uses: the forward additionally emits the
  * ReLU mask as one bit per activation, and the backward consumes that mask instead of re-reading
  * the float32 activation (51 200 B per frame).

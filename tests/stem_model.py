@@ -1,11 +1,12 @@
 """NumPy model of the arithmetic of the derl_b200 stem kernels (test infrastructure).
 
-K6 / K6t (csrc/stem.cu, csrc/stem_tc.cu) and K7t (csrc/stem_bwd_tc.cu) evaluate the reference's
+K6t (csrc/stem_tc.cu) and K7t (csrc/stem_bwd_tc.cu) evaluate the reference's
 first layer (derl/models.py:102-103,117-123: `.float()/255` -> nn.Conv2d(4, 32, 8, 4) -> nn.ReLU)
 and its backward on the INT8 tensor cores: one operand (the uint8 frame) is exact, the other
 (weights forward, the masked gradient backward) is expressed as two signed 8-bit digit planes,
 value ~= s * (q1 + q2 / 254).  This module restates that number format step by step so that
-its error bounds can be pinned on the CPU against the float64 formulation of the reference.
+its error bounds can be pinned on the CPU against the float64 formulation of the reference; the
+forward restates K6t's arithmetic exactly, so the GPU tests compare the kernel with it bit for bit.
 """
 import numpy as np
 
@@ -23,7 +24,7 @@ def patches(frames):
 
 
 def weight_digits(weight):
-  """csrc/stem.cu (digit planes of the weights): per output channel s = max|w| / 127,
+  """csrc/stem_tc.cu (digit planes of the weights): per output channel s = max|w| / 127,
   q1 = rint(w / s), q2 = clamp(rint((w - q1 s) * 254 / s), +-127), all in float32."""
   w = weight.astype(F)
   m = np.abs(w).reshape(w.shape[0], -1).max(1)
@@ -35,16 +36,22 @@ def weight_digits(weight):
   return s, q1.astype(np.int64), q2.astype(np.int64)
 
 
-def stem_forward(frames, weight, bias):
-  """K6: relu(conv(frames / 255, weight, bias, stride 4)) -> float32 [B,20,20,32]."""
+def stem_forward(frames, weight, bias, chunk=64):
+  """K6t: relu(conv(frames / 255, weight, bias, stride 4)) -> float32 [B,20,20,32], bit for bit:
+  both = acc1 * 254 + acc2 (exact), y = relu(float(both) * float32(s / 64770) + bias), each step
+  rounded to float32 as in the kernel's epilogue.  The digit sums run as a float32 matmul, which
+  is exact: every partial sum is an integer of magnitude <= 256 * 255 * 127 < 2^24."""
   s, q1, q2 = weight_digits(weight)
-  x = patches(frames)
-  acc1 = np.einsum("bijklc,nckl->bijn", x, q1)          # exact integers (|.| < 2^24)
-  acc2 = np.einsum("bijklc,nckl->bijn", x, q2)
-  scale = (s * F(1.0 / 255.0)).astype(F)
-  y = (acc1.astype(F) + acc2.astype(F) * F(1.0 / 254.0)).astype(F) * scale
-  y = y.astype(F) + bias.astype(F)
-  return np.maximum(y, F(0)).astype(F), (s, q1, q2)
+  w = np.concatenate([q1, q2]).transpose(2, 3, 1, 0).reshape(256, 64).astype(F)   # [(kh,kw,c), n']
+  es = (s / F(64770)).astype(F)
+  b = bias.astype(F)
+  out = np.empty((frames.shape[0], 20, 20, 32), F)
+  for i in range(0, frames.shape[0], chunk):
+    acc = (patches(frames[i:i + chunk]).reshape(-1, 256).astype(F) @ w).astype(np.int64)
+    both = acc[:, :32] * 254 + acc[:, 32:]
+    y = (both.astype(F) * es).astype(F) + b
+    out[i:i + chunk] = np.maximum(y, F(0)).reshape(-1, 20, 20, 32)
+  return out, (s, q1, q2)
 
 
 def gradient_digits(masked):

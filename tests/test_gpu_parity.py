@@ -718,7 +718,7 @@ def test_graph_replayed_micro_batched_update_with_fused_gather(golden, tf32):
 # losses.  Two different things are bounded:
 #  * the FIRST loss is a pure forward pass on identical parameters — it measures the arithmetic
 #    itself: TF32 tensor-core conv/GEMM (10-bit mantissa operands, fp32 accumulation) plus the
-#    INT8 two-digit stem K6 (operand residual <= 1/508 of a channel's scale).  Measured on B200
+#    INT8 two-digit stem K6t (operand residual <= 1/508 of a channel's scale).  Measured on B200
 #    (profiles/r02_tf32_parity.txt): 9.2e-5 relative (6.2e-5 for the TF32 library path); bound 5e-4.
 #  * later losses follow 1..7 Adam steps.  Adam's update lr * m / (sqrt(v) + eps) is sign-like in
 #    its first steps, so a 1e-3 relative gradient perturbation (TF32's operand rounding) moves
@@ -860,9 +860,10 @@ def test_space_to_depth_kernel_and_its_inverse(dtype):
 
 @pytest.mark.parametrize("dtype", [torch.float32, torch.bfloat16])
 def test_stem_conv_kernel_vs_float32_convolution(dtype):
-  """K6: conv 8x8/4 + bias + ReLU straight from uint8 frames (bf16 MMA, weights hi + lo) against
-  the reference formulation in float32 (`.float()/255` -> conv2d -> relu, TF32 off).  The
-  split keeps ~16 weight bits: 1e-4 relative on activations of O(1) (bf16 output: bf16 rounding)."""
+  """K6t: conv 8x8/4 + bias + ReLU straight from uint8 frames (INT8 MMA, weights as two signed
+  8-bit digit planes) against the reference formulation in float32 (`.float()/255` -> conv2d ->
+  relu, TF32 off).  The digits keep each weight to 1.6e-5 of its channel's largest: 1e-4 relative
+  on activations of O(1) (bf16 output: bf16 rounding)."""
   torch.backends.cudnn.allow_tf32 = False
   gen = torch.Generator(device=DEV).manual_seed(12)
   weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.1
@@ -883,7 +884,7 @@ def test_stem_conv_kernel_vs_float32_convolution(dtype):
 
 
 def test_stem_forward_kernels_with_fused_row_gather_are_bit_identical():
-  """K6 / K6t with `rows`: frame i of the batch is source[rows[i]], pulled straight out of the
+  """K6t with `rows`: frame i of the batch is source[rows[i]], pulled straight out of the
   resident rollout (SURVEY §8f rank 2).  Same bytes in, deterministic kernels: bit-identical to
   running them on the materialised gather, for both output layouts, with repeated rows (the
   backward's `rows` is checked by test_stem_tcgen05_pair_against_its_number_format)."""
@@ -891,7 +892,7 @@ def test_stem_forward_kernels_with_fused_row_gather_are_bit_identical():
   weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.05
   bias = torch.randn(32, device=DEV, generator=gen) * 0.1
   source = torch.randint(0, 256, (97, 84, 84, 4), device=DEV, dtype=torch.uint8, generator=gen)
-  for count in (1, 5, 300):   # 300 > 97: rows repeat; > 296 CTAs of K6: second frames per CTA
+  for count in (1, 5, 300):   # 300 > 97: rows repeat; > 148 CTAs (one per SM): second frames per CTA
     rows = torch.randint(0, 97, (count,), device=DEV, generator=gen)
     dense = source[rows]
     for blk in (1, 2):
@@ -976,7 +977,7 @@ def test_fused_gather_minibatches_and_update_match_the_materialised_pipeline():
 
 
 def test_stem_autograd_matches_cudnn_path():
-  """NatureCNN with the K6 stem (TF32 allowed) vs the cuDNN stem: outputs and all parameter
+  """NatureCNN with the K6t stem (TF32 allowed) vs the cuDNN stem: outputs and all parameter
   gradients agree to TF32-level tolerance; the stem weight gradient lands in [32,4,8,8] layout."""
   torch.manual_seed(0)
   model = d.NatureCNNModel([4, 1])
@@ -1011,7 +1012,7 @@ def test_space_to_depth_first_conv_equals_plain_formulation():
   for s2d, fused in ((True, True), (True, False), (False, False), ("hidden", True)):
     d.NatureCNNBase.space_to_depth, d.NatureCNNBase.fused_conv_relu = bool(s2d), fused
     d.NatureCNNBase.space_to_depth_hidden = s2d == "hidden"
-    model.zero_grad()  # (TF32 is off here, so the K6 stem is not in play: cuDNN float32 stem)
+    model.zero_grad()  # (TF32 is off here, so the K6t stem is not in play: cuDNN float32 stem)
     logits, values = model(frames)
     (logits.square().sum() + values.sum()).backward()
     outs[s2d, fused] = (logits.detach().clone(), values.detach().clone(),
@@ -1379,24 +1380,30 @@ def test_fused_mlp_plan_rejects_what_it_does_not_model():
 # =============================================================================== K6t: tcgen05 stem
 @pytest.mark.parametrize("batch", [1, 3, 149, 700])
 @pytest.mark.parametrize("out_block", [1, 2])
-def test_stem_tcgen05_kernel_is_bit_identical_to_the_mma_sync_kernel(monkeypatch, batch, out_block):
+def test_stem_forward_kernel_against_its_number_format(batch, out_block):
   """K6t (csrc/stem_tc.cu: tcgen05.mma kind::i8, accumulators in tensor memory, TMA-permuted
-  frame tile as a no-swizzle K-major operand) computes the same exact int32 sums and the same
-  fp32 epilogue as the legacy mma.sync kernel, so the two must agree bit for bit — with and
-  without the fused gather (`rows`, repeated indices included) — and both stay within 1e-4 of
-  the activation scale of the float32 convolution (derl/models.py:102-103,117-123)."""
+  frame tile as a no-swizzle K-major operand) computes exact int32 digit sums and a separately
+  rounded fp32 epilogue, so its float32 output equals the NumPy restatement of that arithmetic
+  (tests/stem_model.py) bit for bit — with and without the fused gather (`rows`, repeated indices
+  included).  The bf16 output is the float32 one rounded to nearest even, and the float32 output
+  stays within 1e-4 of the activation scale of the float32 convolution
+  (derl/models.py:102-103,117-123)."""
   gen = torch.Generator(device=DEV).manual_seed(batch)
   weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.1
   bias = torch.randn(32, device=DEV, generator=gen) * 0.1
   frames = torch.randint(0, 256, (batch, 84, 84, 4), dtype=torch.uint8, device=DEV, generator=gen)
   rows = torch.randint(0, batch, (batch + 3,), device=DEV, generator=gen)
+  model, _ = stem_model.stem_forward(frames.cpu().numpy(), weight.cpu().numpy(),
+                                     bias.cpu().numpy())
+  model = torch.from_numpy(model).to(DEV)
   for sel in (None, rows):
-    monkeypatch.delenv("DERL_STEM_MMA_SYNC", raising=False)
-    new = K.stem_conv_relu(frames, weight, bias, torch.float32, out_block, sel)
-    monkeypatch.setenv("DERL_STEM_MMA_SYNC", "1")
-    old = K.stem_conv_relu(frames, weight, bias, torch.float32, out_block, sel)
-    assert torch.equal(new, old), f"rows={'yes' if sel is not None else 'no'}"
-  monkeypatch.delenv("DERL_STEM_MMA_SYNC", raising=False)
+    want = model if sel is None else model[sel]
+    if out_block == 2:
+      want = K.space_to_depth(want, 2, False)
+    got = K.stem_conv_relu(frames, weight, bias, torch.float32, out_block, sel)
+    assert torch.equal(got, want), f"rows={'yes' if sel is not None else 'no'}"
+    half = K.stem_conv_relu(frames, weight, bias, torch.bfloat16, out_block, sel)
+    assert torch.equal(half, got.to(torch.bfloat16)), f"bf16, rows={'yes' if sel is not None else 'no'}"
   if out_block == 1:
     torch.backends.cudnn.allow_tf32 = False
     try:
@@ -1411,17 +1418,19 @@ def test_stem_tcgen05_kernel_is_bit_identical_to_the_mma_sync_kernel(monkeypatch
 def test_stem_tcgen05_kernel_is_deterministic_under_repetition():
   """Stress for the mbarrier rings of K6t (TMA -> MMA -> two epilogue groups -> TMA store): 30
   launches over batch sizes that leave CTAs with 0, 1 or many frames must all give the first
-  launch's bytes (a race in the pipeline shows up as a sporadic difference)."""
+  launch's bytes (a race in the pipeline shows up as a sporadic difference), for the float32 and
+  the bf16 staging layouts."""
   gen = torch.Generator(device=DEV).manual_seed(9)
   weight = torch.randn(32, 4, 8, 8, device=DEV, generator=gen) * 0.1
   bias = torch.randn(32, device=DEV, generator=gen) * 0.1
   for batch in (5, 148, 151, 2000):
     frames = torch.randint(0, 256, (batch, 84, 84, 4), dtype=torch.uint8, device=DEV,
                            generator=gen)
-    ref = K.stem_conv_relu(frames, weight, bias, torch.float32, 2, None)
-    for _ in range(30):
-      again = K.stem_conv_relu(frames, weight, bias, torch.float32, 2, None)
-      assert torch.equal(again, ref)
+    for dtype in (torch.float32, torch.bfloat16):
+      ref = K.stem_conv_relu(frames, weight, bias, dtype, 2, None)
+      for _ in range(30):
+        again = K.stem_conv_relu(frames, weight, bias, dtype, 2, None)
+        assert torch.equal(again, ref)
 
 
 def _expected_relu_mask(plain_out):

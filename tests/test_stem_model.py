@@ -1,8 +1,8 @@
-"""Pins, on the CPU, the number format the INT8 stem kernels (K6 forward, K7t backward) use
+"""Pins, on the CPU, the number format the INT8 stem kernels (K6t forward, K7t backward) use
 against the float64 formulation of the reference's first layer (derl/models.py:102-103,
 117-123).  The GPU parity tests check the kernels against float32 convolutions; these tests
 check the format itself: digit ranges, the <= s/508 residual, and the end-to-end error of the
-activations and of the weight gradient — the claims made in DESIGN.md §3 K6 / K7t."""
+activations and of the weight gradient — the claims made in DESIGN.md §3 K6t / K7t."""
 import numpy as np
 
 from stem_model import gradient_digits, patches, stem_backward, stem_forward, weight_digits

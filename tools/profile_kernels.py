@@ -90,11 +90,9 @@ def main():
   timed("stem_conv_relu_mask 32768 blk2 (K6t)",
         lambda: K.stem_conv_relu_mask(obs[:32768], wstem, bstem, 2),
         32768 * (28224 + 400 * 32 * 4.0 + 1792))
-  os.environ["DERL_STEM_MMA_SYNC"] = "1"
-  timed("stem_conv_relu 32768 blk2 (K6, mma.sync)",
-        lambda: K.stem_conv_relu(obs[:32768], wstem, bstem, torch.float32, 2),
-        32768 * (28224 + 400 * 32 * 4.0))
-  os.environ.pop("DERL_STEM_MMA_SYNC")
+  timed("stem_conv_relu 32768 bf16 blk2 (K6t)",
+        lambda: K.stem_conv_relu(obs[:32768], wstem, bstem, torch.bfloat16, 2),
+        32768 * (28224 + 400 * 32 * 2.0))
   act, relu_mask = K.stem_conv_relu_mask(obs[:32768], wstem, bstem, 2)
   act = act.permute(0, 3, 1, 2)
   gact = torch.randn_like(act) * 1e-3

@@ -1,5 +1,5 @@
 """One small launch of every kernel with an mbarrier / TMA pipeline (K1 TMA scan, K2 row gather,
-K6 / K6t stem forward, K7t stem backward), for `compute-sanitizer --tool racecheck` (shared-
+K6t stem forward, K7t stem backward), for `compute-sanitizer --tool racecheck` (shared-
 memory hazards) or `--tool memcheck` / `--tool synccheck`:
 
     compute-sanitizer --tool racecheck python tools/race_targets.py [repeats]
@@ -30,12 +30,10 @@ def main():
     frames = torch.randint(0, 256, (400, 84, 84, 4), dtype=torch.uint8, device="cuda", generator=gen)
     perm = torch.randperm(400, device="cuda", generator=gen)
     K.gather_rows(frames, perm, 3, 390)
-    # K6 / K6t / K7t
+    # K6t (bf16, float32 with mask, float32) / K7t
     weight = torch.randn(32, 4, 8, 8, device="cuda", generator=gen) * 0.1
     bias = torch.randn(32, device="cuda", generator=gen) * 0.1
-    os.environ["DERL_STEM_MMA_SYNC"] = "1"
-    K.stem_conv_relu(frames, weight, bias, torch.float32, 2, None)
-    os.environ.pop("DERL_STEM_MMA_SYNC")
+    K.stem_conv_relu(frames, weight, bias, torch.bfloat16, 2, None)
     out, mask = K.stem_conv_relu_mask(frames, weight, bias, 2, perm)
     K.stem_conv_relu(frames, weight, bias, torch.float32, 1, None)
     grad = torch.randn(400, 128, 10, 10, device="cuda", generator=gen).contiguous(
