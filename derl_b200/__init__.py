@@ -11,7 +11,7 @@ from .alg import (A2C, A2CLoss, Alg, GraphedTrainer, Loss, PPO, PPOLoss, Trainer
 from .anneal import AnnealingVariable, LinearAnneal
 from .models import MLP, MuJoCoModel, NatureCNNBase, NatureCNNModel, make_model, orthogonal_init
 from .policies import ActorCriticPolicy, Policy
-from .runners import (EnvRunner, FrameStackPacker, FrameStacks, GAE, IterateWithMinibatches,
-                      MergeTimeBatch, NormalizeAdvantages, PeriodicSummaries, RunnerWrapper,
-                      SyntheticRolloutRunner, Take, TransformInteractions, make_frame_stack_rollout,
+from .runners import (DeviceFrameStackPacker, EnvRunner, FrameStackPacker, FrameStacks, GAE,
+                      IterateWithMinibatches, MergeTimeBatch, NormalizeAdvantages,
+                      PeriodicSummaries, RunnerWrapper, SyntheticRolloutRunner, Take, TransformInteractions, make_frame_stack_rollout,
                       make_ppo_runner, make_rollout, ppo_runner_wrap)

@@ -8,7 +8,7 @@ import os
 
 _PKG = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_PKG, "libderl_b200.so")
-ABI_VERSION = 6
+ABI_VERSION = 7
 
 GAE_AUTO, GAE_DIRECT, GAE_TMA = 0, 1, 2
 GAE_STATS = 3
@@ -35,6 +35,9 @@ SIGNATURES = {
                                             _ptr]),
     "derl_b200_gather_frame_stacks": (_int, [_ptr, _i64, _i64, _i64, _ptr, _i64, _i64, _ptr, _i64,
                                              _i64, _ptr, _ptr]),
+    "derl_b200_pack_frame_stacks_workspace_bytes": (_size, [_i64, _i64]),
+    "derl_b200_pack_frame_stacks": (_int, [_ptr, _ptr, _ptr, _i64, _i64, _i64, _i64, _ptr, _i64,
+                                           _ptr, _ptr, _ptr, _size, _ptr]),
     "derl_b200_gather_columns": (_int, [_int, _ptr, _ptr, _ptr, _ptr, _i64, _i64, _int, _ptr,
                                         _ptr, _size, _ptr]),
     "derl_b200_ppo_loss_workspace_bytes": (_size, [_i64]),

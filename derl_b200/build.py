@@ -15,7 +15,7 @@ CSRC = os.path.join(PKG_DIR, "csrc")
 INCLUDE = os.path.join(REPO_DIR, "include")
 LIB_PATH = os.path.join(PKG_DIR, "libderl_b200.so")
 STAMP_PATH = os.path.join(PKG_DIR, ".libderl_b200.stamp")
-SOURCES = ("abi.cu", "gae.cu", "gather.cu", "frame_stacks.cu", "ppo_loss.cu", "frames.cu", "relu_bwd.cu", "stem_tc.cu", "stem_bwd_tc.cu", "mlp_update.cu", "heads.cu",
+SOURCES = ("abi.cu", "gae.cu", "gather.cu", "frame_stacks.cu", "frame_pack.cu", "ppo_loss.cu", "frames.cu", "relu_bwd.cu", "stem_tc.cu", "stem_bwd_tc.cu", "mlp_update.cu", "heads.cu",
            "host_api.cu")
 NVCC_FLAGS = (
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -254,6 +254,48 @@ def _(frames, index, perm, start, count):
   return frames.new_empty((count,) + tuple(frames.shape[1:]) + (index.shape[1],))
 
 
+# --------------------------------------------------------------------------- K11: frame packing
+@torch.library.custom_op("derl_b200::pack_frame_stacks", mutates_args=("pool", "state", "ids"),
+                         device_types="cuda")
+def pack_frame_stacks(stacks: Tensor, prev_stacks: Optional[Tensor], prev_ids: Optional[Tensor],
+                      pool: Tensor, state: Tensor, ids: Tensor) -> None:
+  """Packs one step of stacks [N, H, W, k] uint8 into the planes pool [capacity, H, W] exactly as
+  FrameStackPacker.pack does: writes the step's int32 [N, k] plane ids into `ids`, appends the new
+  planes to `pool` and advances state = int64 {plane count, overflow flag}, all on the device.
+  prev_stacks / prev_ids are the previous step's stacks and ids (None on a rollout's first step).
+  A step that would not fit in `pool` sets the (sticky) overflow flag instead of writing."""
+  _dense(stacks, "stacks", (torch.uint8,))
+  _dense(pool, "pool", (torch.uint8,))
+  _dense(state, "state", (torch.int64,))
+  _dense(ids, "ids", (torch.int32,))
+  _need(stacks.dim() == 4, f"stacks must be [N, H, W, k], got {tuple(stacks.shape)}")
+  nenvs, height, width, k = stacks.shape
+  _need(pool.dim() == 3 and tuple(pool.shape[1:]) == (height, width),
+        f"pool must be [capacity, {height}, {width}], got {tuple(pool.shape)}")
+  _need(state.numel() == 2, "state must hold {count, overflow}")
+  _need(tuple(ids.shape) == (nenvs, k), f"ids must be [{nenvs}, {k}], got {tuple(ids.shape)}")
+  _need((prev_stacks is None) == (prev_ids is None), "prev_stacks and prev_ids go together")
+  if prev_stacks is not None:
+    _dense(prev_stacks, "prev_stacks", (torch.uint8,))
+    _dense(prev_ids, "prev_ids", (torch.int32,))
+    _need(prev_stacks.shape == stacks.shape and tuple(prev_ids.shape) == (nenvs, k),
+          "the previous step must have the same shape as this one")
+  tensors = [stacks, pool, state, ids] + ([prev_stacks, prev_ids] if prev_stacks is not None else [])
+  _need(all(t.device == stacks.device for t in tensors), "all tensors must share a device")
+  lib = _lib.load()
+  ws_bytes = lib.derl_b200_pack_frame_stacks_workspace_bytes(nenvs, k)
+  ws = torch.empty(max(ws_bytes, 16), dtype=torch.uint8, device=stacks.device)
+  with _device_of(stacks, "pack_frame_stacks"):
+    _lib.check(lib.derl_b200_pack_frame_stacks(
+        _p(stacks), _p(prev_stacks), _p(prev_ids), nenvs, height, width, k, _p(pool),
+        pool.shape[0], _p(state), _p(ids), _p(ws), ws_bytes, _stream(stacks)), "pack_frame_stacks")
+
+
+@pack_frame_stacks.register_fake
+def _(stacks, prev_stacks, prev_ids, pool, state, ids):
+  return None
+
+
 @torch.library.custom_op("derl_b200::gather_columns", mutates_args=(), device_types="cuda")
 def gather_columns(columns: List[Tensor], perm: Tensor, start: int, count: int,
                    moments_col: int = -1) -> List[Tensor]:

@@ -1,5 +1,5 @@
 from .env_runner import EnvRunner, RunnerWrapper
-from .frame_stacks import FrameStackPacker, FrameStacks
+from .frame_stacks import DeviceFrameStackPacker, FrameStackPacker, FrameStacks
 from .onpolicy import (TransformInteractions, IterateWithMinibatches, gather_minibatch,
                        ppo_runner_wrap, make_ppo_runner)
 from .summary import PeriodicSummaries

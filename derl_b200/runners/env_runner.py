@@ -11,7 +11,7 @@ from abc import ABC, abstractmethod
 import numpy as np
 import torch
 
-from .frame_stacks import FrameStackRollout
+from .frame_stacks import DeviceFrameStackPacker, FrameStackRollout
 
 _FORWARDED = frozenset(("env", "policy", "horizon", "nsteps", "step_count", "nenvs",
                         "is_exhausted"))
@@ -78,9 +78,11 @@ class EnvRunner:
 
   `pack_frames` (extension, default False): `observations` is yielded as a
   `runners.frame_stacks.FrameStacks` — every frame plane stored once plus a per-sample stack
-  index, packed on the host one step at a time — instead of stacked arrays: about a quarter of the
-  bytes for 4-frame Atari stacks.  Without `resident_device` the planes are in pinned host memory
-  (TransformInteractions uploads them); with it they are copied to the device step by step.
+  index, packed one step at a time — instead of stacked arrays: about a quarter of the bytes for
+  4-frame Atari stacks.  Without `resident_device` the host packs (FrameStackPacker) and the
+  planes stay in pinned host memory (TransformInteractions uploads them).  With it each step's
+  stacks are copied to the device and packed there (DeviceFrameStackPacker, kernel K11): planes
+  and index are born in HBM, and the host does no more per step than the stacked resident route.
   `state["latest_observations"]` stays stacked in both modes.
   """
 
@@ -97,6 +99,7 @@ class EnvRunner:
     self.step_count = 0
     self.episode_length = 0
     self._resident = None
+    self._frame_packer = None
 
   @property
   def nenvs(self):
@@ -120,7 +123,11 @@ class EnvRunner:
           self._resident = _ResidentRollout(self.horizon, self.resident_device)
         resident = self._resident
         resident.begin()
-      frames = FrameStackRollout(self.horizon, self.resident_device) if self.pack_frames else None
+      frames = None
+      if self.pack_frames:
+        if self.resident_device is not None and self._frame_packer is None:
+          self._frame_packer = DeviceFrameStackPacker(self.resident_device, self.horizon)
+        frames = FrameStackRollout(self.horizon, self.resident_device, self._frame_packer)
 
       def put(key, val, step):
         if resident is not None and key == "next_observations":

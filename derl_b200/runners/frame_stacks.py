@@ -16,6 +16,7 @@ so everything downstream of the gather is unchanged.
 
   FrameStacks        the column: enough of the array interface for the runner wrappers
   FrameStackPacker   host packer, one env step [N, H, W, k] at a time (NumPy)
+  DeviceFrameStackPacker  the same packing on the GPU (K11), planes in a device pool
   FrameStackRollout  one rollout's observations collected by EnvRunner(pack_frames=True)
   unpack             NumPy restatement of the format (frames, index) -> stacked array
 """
@@ -228,46 +229,171 @@ class FrameStackPacker:
     return ids
 
 
+class DeviceFrameStackPacker:
+  """FrameStackPacker on the GPU (K11, torch.ops.derl_b200.pack_frame_stacks): the same ids and
+  plane bytes for the same steps, with the planes in a device pool and no host synchronisation
+  per step.
+
+  `pack(obs, out=None)` takes a NumPy [N, H, W, k] uint8 step or a CUDA uint8 tensor of that
+  shape and writes the int32 [N, k] ids into `out` (a device row, e.g. one row of a rollout's
+  index) or returns them as a new device tensor.  A NumPy step goes through one of two pinned
+  staging slots (rewritten only once the slot's previous copy has completed) and an asynchronous
+  copy into one of two device stack buffers, which hold the current and the previous step; a CUDA
+  step is copied device to device, since the caller may reuse its tensor.  Everything runs on the
+  current stream, and the buffers are allocated once and reused across rollouts.
+
+  The plane count stays on the device.  After each step it is copied into a pinned per-step ring
+  and an event is recorded; before a step the pool is grown (stream-ordered device copy) if the
+  latest count known to have arrived, plus N*k planes for every step since, could exceed it.
+  `reset()` starts a rollout with a fresh pool of `horizon*N + N*(k-1)` planes (the standard
+  stacking case) plus N*k headroom; `finish()` reads the count once, raises RuntimeError if a step
+  overflowed the pool, and returns the planes [count, H, W].
+  """
+
+  def __init__(self, device, horizon):
+    self.device = torch.device(device)
+    self.horizon = max(int(horizon), 1)
+    self._shape = None
+    self._stacks = None       # device uint8 [2, N, H, W, k]: current and previous step
+    self._staging = None      # pinned uint8 [2, N, H, W, k]
+    self._staged = [None, None]   # event of each staging slot's last copy
+    self._state = torch.zeros(2, dtype=torch.int64, device=self.device)
+    self._counts = torch.zeros(self.horizon, dtype=torch.int64, pin_memory=True)
+    self._count_events = [torch.cuda.Event() for _ in range(self.horizon)]
+    self.reset()
+
+  def reset(self):
+    """Start a rollout: no previous step, count 0, a new pool (the old one now belongs to the
+    FrameStacks that `finish` returned)."""
+    self._pool, self._prev_ids = None, None
+    self._steps = 0
+    self._known = (-1, 0)     # (step, plane count after it) last read from the pinned ring
+    self._pending = []        # steps whose count copy has not been read yet, oldest first
+    self._state.zero_()
+
+  def _buffers(self, shape):
+    if self._shape == shape:
+      return
+    if self._steps:
+      raise ValueError(f"step shape {shape} differs from the previous step's {self._shape}")
+    self._shape = shape
+    self._stacks = torch.empty((2,) + shape, dtype=torch.uint8, device=self.device)
+    self._staging, self._staged = None, [None, None]
+
+  def _bound(self, nk):
+    """Upper bound of the plane count after the step about to be packed."""
+    while self._pending and self._count_events[self._pending[0] % self.horizon].query():
+      step = self._pending.pop(0)
+      self._known = (step, int(self._counts[step % self.horizon]))
+    step, count = self._known
+    return count + (self._steps - step) * nk
+
+  def _reserve(self, need, nk):
+    cap = 0 if self._pool is None else self._pool.shape[0]
+    if need <= cap:
+      return
+    if self._pool is None:
+      nenvs, k = self._shape[0], self._shape[-1]
+      need = max(need, self.horizon * nenvs + nenvs * (k - 1) + nk)
+    grown = torch.empty((max(need, cap * 3 // 2),) + self._shape[1:3], dtype=torch.uint8,
+                        device=self.device)
+    if cap:
+      used = min(cap, self._bound(nk) - nk)   # the count before this step is at most this
+      grown[:used].copy_(self._pool[:used])
+    self._pool = grown
+
+  def pack(self, obs, out=None):
+    """Appends one step; returns its int32 [N, k] plane ids (a device tensor, `out` if given)."""
+    if isinstance(obs, torch.Tensor) and obs.is_cuda:
+      src = obs
+    else:
+      src = np.ascontiguousarray(obs)
+    if src.dtype not in (np.uint8, torch.uint8) or src.ndim != 4:
+      raise TypeError(f"expected uint8 [N, H, W, k] observations, got {src.dtype} "
+                      f"{tuple(src.shape)}")
+    shape = tuple(src.shape)
+    self._buffers(shape)
+    nenvs, k = shape[0], shape[-1]
+    slot = self._steps % 2
+    cur = self._stacks[slot]
+    if isinstance(src, torch.Tensor):
+      cur.copy_(src)
+    else:
+      if self._staging is None:
+        self._staging = torch.empty((2,) + shape, dtype=torch.uint8, pin_memory=True)
+      if self._staged[slot] is not None:
+        self._staged[slot].synchronize()
+      np.copyto(self._staging[slot].numpy(), src)
+      cur.copy_(self._staging[slot], non_blocking=True)
+      self._staged[slot] = torch.cuda.current_stream(self.device).record_event()
+    nk = nenvs * k
+    self._reserve(self._bound(nk), nk)
+    if out is not None and self._prev_ids is not None and \
+        out.data_ptr() == self._prev_ids.data_ptr():
+      raise ValueError("out must not be the previous step's ids: the kernel reads them")
+    ids = out if out is not None else torch.empty((nenvs, k), dtype=torch.int32,
+                                                  device=self.device)
+    prev = self._stacks[1 - slot] if self._prev_ids is not None else None
+    _K.pack_frame_stacks(cur, prev, self._prev_ids, self._pool, self._state, ids)
+    ring = self._steps % self.horizon
+    if len(self._pending) == self.horizon:     # the ring slot is still in flight
+      self._count_events[ring].synchronize()
+      self._bound(nk)
+    self._counts[ring].copy_(self._state[0], non_blocking=True)
+    self._count_events[ring].record(torch.cuda.current_stream(self.device))
+    self._pending.append(self._steps)
+    self._prev_ids = ids
+    self._steps += 1
+    return ids
+
+  def finish(self):
+    """The planes packed since `reset`: uint8 [count, H, W] on the device (one host read)."""
+    count, overflow = self._state.tolist()
+    if overflow:
+      raise RuntimeError("frame-plane pool overflowed: a step needed more planes than the pool "
+                         "holds, so this rollout's frames are incomplete")
+    if self._pool is None:
+      raise RuntimeError("nothing was packed since reset()")
+    return self._pool[:count]
+
+
 class FrameStackRollout:
   """`observations` of one EnvRunner rollout, packed as it is collected.
 
-  device None: planes and index accumulate in host memory (pinned when CUDA is available);
-  `finish` returns a host FrameStacks (TransformInteractions uploads it).  device given: every step's new planes and
-  index row are also copied asynchronously into device buffers from the pinned host arrays (as
-  `_ResidentRollout.put` does for the other columns).  The host knows each step's plane count,
-  so the device pool grows by a device-side copy, never by a sync.
+  device None: FrameStackPacker packs on the host; planes and index accumulate in host memory
+  (pinned when CUDA is available) and `finish` returns a host FrameStacks (TransformInteractions
+  uploads it).  device given: a DeviceFrameStackPacker (`packer`, reused across rollouts when the
+  caller passes one) packs on the GPU, writing every step's ids straight into the device index;
+  `finish` returns a device FrameStacks.
   """
 
-  def __init__(self, horizon, device=None):
+  def __init__(self, horizon, device=None, packer=None):
     self.horizon = horizon
     self.device = None if device is None else torch.device(device)
-    self.packer, self.index = None, None
-    self._dev_frames, self._dev_index = None, None
+    self.packer, self.index = packer, None
+    self._dev_index = None
 
   def put(self, step, obs):
-    obs = np.asarray(obs)
+    if not isinstance(obs, torch.Tensor):
+      obs = np.asarray(obs)
+    if self.device is not None:
+      if self._dev_index is None:
+        nenvs, k = obs.shape[0], obs.shape[-1]
+        if self.packer is None:
+          self.packer = DeviceFrameStackPacker(self.device, self.horizon)
+        self.packer.reset()
+        self._dev_index = torch.empty((self.horizon, nenvs, k), dtype=torch.int32,
+                                      device=self.device)
+      self.packer.pack(obs, out=self._dev_index[step])
+      return
     if self.packer is None:
       nenvs, k = obs.shape[0], obs.shape[-1]
       pinned = torch.cuda.is_available()   # page-locked only where a GPU will read it
       self.packer = FrameStackPacker(self.horizon * nenvs + nenvs * (k - 1), pinned=pinned)
       self.index = _pinned((self.horizon, nenvs, k), torch.int32, pinned)
-    lo = self.packer.count
     self.index[step].numpy()[...] = self.packer.pack(obs)
-    if self.device is None:
-      return
-    hi = self.packer.count
-    if self._dev_frames is None or self._dev_frames.shape[0] < hi:
-      grown = torch.empty((self.packer.capacity,) + tuple(obs.shape[1:3]), dtype=torch.uint8,
-                          device=self.device)
-      if self._dev_frames is not None and lo:
-        grown[:lo].copy_(self._dev_frames[:lo])
-      self._dev_frames = grown
-      if self._dev_index is None:
-        self._dev_index = torch.empty(self.index.shape, dtype=torch.int32, device=self.device)
-    self._dev_frames[lo:hi].copy_(self.packer.frames[lo:hi], non_blocking=True)
-    self._dev_index[step].copy_(self.index[step], non_blocking=True)
 
   def finish(self):
     if self.device is None:
       return FrameStacks(self.packer.frames, self.index, validate=False)
-    return FrameStacks(self._dev_frames[:self.packer.count], self._dev_index, validate=False)
+    return FrameStacks(self.packer.finish(), self._dev_index, validate=False)

@@ -33,8 +33,10 @@ extern "C" {
  *    derl_b200_stem_conv_relu_mask / derl_b200_stem_backward_masked (tcgen05 stem pair).
  * 5: derl_b200_gather_frame_stacks (minibatch gather out of a frame-plane rollout).
  * 6: derl_b200_stem_backward (the stem backward from the float32 activation) removed:
- *    derl_b200_stem_backward_masked is the stem backward. */
-#define DERL_B200_ABI_VERSION 6
+ *    derl_b200_stem_backward_masked is the stem backward.
+ * 7: derl_b200_pack_frame_stacks / derl_b200_pack_frame_stacks_workspace_bytes (frame-plane
+ *    packing of one env step on the device). */
+#define DERL_B200_ABI_VERSION 7
 
 enum {
   DERL_OK = 0,
@@ -162,6 +164,36 @@ int derl_b200_gather_frame_stacks(const void* frames_dev, int64_t n_frames, int6
                                   int64_t width, const int32_t* index_dev, int64_t n_samples,
                                   int64_t k, const int64_t* perm_dev, int64_t start, int64_t count,
                                   void* dst_dev, void* stream);
+
+/* ------------------------------------------------------------------ K11: frame-stack packing
+ * Packs one env step of stacked observations into the frame-plane format K10 reads, on the
+ * device: FrameStackPacker.pack (derl_b200/runners/frame_stacks.py) is the specification, and for
+ * the same sequence of steps this entry point hands out the same plane ids and writes the same
+ * plane bytes, bit for bit.  Channel k-1 of every stack is a new plane; for c = k-2 ... 0 channel
+ * c of env n reuses the id of channel c+1 of the same stack if their bytes are equal, else the id
+ * of channel c+1 of env n's previous step if those bytes are equal, else it is a new plane.  New
+ * ids are handed out from the running count: channel k-1 of env 0..n-1, then the new planes of
+ * channel k-2 in env order, and so on down to channel 0.
+ *   stacks_dev      uint8 [n, height, width, k]   this step (NHWC stacks)
+ *   prev_stacks_dev uint8 [n, height, width, k]   the previous step, or NULL on a rollout's first
+ *   prev_ids_dev    int32 [n, k]                  the previous step's ids; NULL iff prev_stacks_dev is
+ *   pool_dev        uint8 [capacity, height, width]  the planes; new ones are appended in place
+ *   state_dev       int64 [2]                     {plane count, overflow flag}, read and updated in
+ *                                                 place; zero both to start a rollout
+ *   ids_dev         int32 [n, k] out              this step's plane ids (e.g. one index row)
+ * Nothing is read back to the host and nothing synchronises.  A step whose planes would not fit
+ * in `capacity` writes no plane at or beyond it and no ids: it sets the overflow flag, which is
+ * sticky (every later step does nothing) and must be checked by the caller at the end.
+ * k == 4 with height*width % 16 == 0 and 16-byte aligned stacks / prev_stacks / pool takes the
+ * vectorised path; any 1 <= k <= 32 and any height x width the plain one.  capacity and n*k must
+ * fit int32.  workspace_dev >= derl_b200_pack_frame_stacks_workspace_bytes(n, k) (scratch; contents
+ * undefined before and after; 0 for a k outside 1..32). */
+size_t derl_b200_pack_frame_stacks_workspace_bytes(int64_t n, int64_t k);
+int derl_b200_pack_frame_stacks(const void* stacks_dev, const void* prev_stacks_dev,
+                                const int32_t* prev_ids_dev, int64_t n, int64_t height,
+                                int64_t width, int64_t k, void* pool_dev, int64_t capacity,
+                                int64_t* state_dev, int32_t* ids_dev, void* workspace_dev,
+                                size_t workspace_bytes, void* stream);
 
 /* ------------------------------------------------------------------ K3: fused PPO loss
  * Replaces PPOLoss.__call__ (derl/alg/ppo.py:100-108) = policy_loss (:31-64) +

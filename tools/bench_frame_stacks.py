@@ -13,6 +13,16 @@ Arms, each timed with CUDA events in one process, the two forms alternating step
             vs FrameStacks (frames + index uploaded by one copy each)
   capacity  32 768 envs x 128 steps as FrameStacks on one GPU: update time, peak allocation
   packer    FrameStackPacker.pack per step at N = 4096 (host CPU time)
+  device_packer  DeviceFrameStackPacker (K11) at N = 4096, 84x84x4: host time per `pack` call
+            (NumPy step: pinned staging copy + launches), K11 device time per step from CUDA events
+            (launches queued behind a sleep kernel, so no host gap is timed; L2 overwritten with
+            256 MB before every step, so the previous step's stacks are not L2-resident), its
+            algorithmic bytes and share of HBM peak, and the H2D bytes per step
+  collect   seconds per 128-step rollout of EnvRunner(resident_device=...) at N = 4096 on a cheap
+            stacking env that shifts in frames from a pre-generated bank: stacked vs
+            pack_frames=True (device packing), alternating; the host-packing route
+            (pack_frames=True without resident_device) once; and the env + policy alone
+    python tools/bench_frame_stacks.py --pack-only     # packer, device_packer and collect arms
 The GPU name, power limit and SM clock are read in the same run.
 """
 import argparse
@@ -60,6 +70,152 @@ def packer_arm(nenvs, steps, seed=0):
           "ms_per_step_max": float(np.max(steady)) * 1e3, "first_step_ms": times[0] * 1e3,
           "planes": packer.count, "threads": torch.get_num_threads(),
           "what": "host CPU time of FrameStackPacker.pack on [N, 84, 84, 4] uint8 steps"}
+
+
+class BankEnv:
+  """Batched env with baselines-style 84x84x4 stacks that shifts in one frame per step from a
+  pre-generated bank, so that collection timings are not dominated by an emulator."""
+
+  def __init__(self, nenvs, bank=8, seed=0):
+    rng = np.random.default_rng(seed)
+    self.bank = rng.integers(0, 256, (bank, nenvs, 84, 84), dtype=np.uint8)
+    self.nenvs, self.t = nenvs, 0
+    self.unwrapped = self
+    self.stack = None
+
+  def reset(self):
+    self.stack = np.stack([self.bank[i] for i in range(4)], -1)
+    self.t = 4
+    return self.stack
+
+  def step(self, actions):
+    self.stack = np.concatenate([self.stack[..., 1:],
+                                 self.bank[self.t % len(self.bank)][..., None]], -1)
+    self.t += 1
+    return self.stack, np.zeros(self.nenvs, np.float32), np.zeros(self.nenvs, bool), {}
+
+
+class SyncPolicy:
+  """Host outputs read back from the device every step, as a GPU policy's are."""
+
+  def __init__(self, nenvs, device):
+    self.nenvs, self.device = nenvs, device
+
+  def act(self, obs):
+    values = torch.zeros(self.nenvs, device=self.device).cpu().numpy()
+    return {"actions": np.zeros(self.nenvs, np.int64), "values": values}
+
+
+def device_packer_arm(nenvs, steps, peak, peak_kind, device):
+  from derl_b200.runners.frame_stacks import DeviceFrameStackPacker
+  K = torch.ops.derl_b200
+  env = BankEnv(nenvs, seed=3)
+  # a bank of 8 frames makes the stacks periodic in 8 steps: cycling these continues the sequence
+  host_steps = [env.reset()] + [env.step(None)[0] for _ in range(7)]
+  plane = 84 * 84
+  # host time per pack call, NumPy input (the EnvRunner route); the device is drained each step,
+  # as policy.act does in EnvRunner, so the staging slot never waits
+  packer = DeviceFrameStackPacker(device, steps)
+  host_ms = []
+  for i in range(steps):
+    t0 = time.perf_counter()
+    packer.pack(host_steps[i % len(host_steps)])
+    host_ms.append((time.perf_counter() - t0) * 1e3)
+    torch.cuda.synchronize()
+  packer.finish()
+  del packer
+  # K11 device time per step: steps on the device, launches queued behind a sleep kernel
+  dev_steps = [torch.from_numpy(s).to(device) for s in host_steps]
+  pool = torch.empty((steps * nenvs * 4 + nenvs * 4, 84, 84), dtype=torch.uint8, device=device)
+  state = torch.zeros(2, dtype=torch.int64, device=device)
+  index = torch.empty((steps, nenvs, 4), dtype=torch.int32, device=device)
+  flush = torch.empty(256 << 20, dtype=torch.uint8, device=device)
+  for _ in range(2):   # warm-up pass, then the timed pass from an empty pool
+    state.zero_()
+    torch.cuda.synchronize()
+    torch.cuda._sleep(200_000_000)
+    events, counts = [], []
+    for i in range(steps):
+      flush.fill_(i & 255)
+      a, b = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+      a.record()
+      prev = dev_steps[(i - 1) % len(dev_steps)] if i else None
+      K.pack_frame_stacks(dev_steps[i % len(dev_steps)], prev, index[i - 1] if i else None, pool,
+                          state, index[i])
+      b.record()
+      events.append((a, b))
+      counts.append(state[0].clone())
+    torch.cuda.synchronize()
+  ms = [a.elapsed_time(b) for a, b in events]
+  counts = [0] + [int(c) for c in counts]
+  new_planes = [counts[i + 1] - counts[i] for i in range(steps)]
+  # steady state: steps after the first (which has no previous step and stores every channel)
+  stack_bytes = nenvs * plane * 4
+  steady = ms[1:]
+  bytes_step = [2 * stack_bytes + 16 * nenvs + new_planes[i] * plane + 16 * nenvs
+                for i in range(1, steps)]
+  t = float(np.median(steady))
+  algo = float(np.median(bytes_step))
+  return {"nenvs": nenvs, "steps": steps, "hw": [84, 84], "k": 4,
+          "host_ms_per_pack": float(np.median(host_ms[1:])),
+          "host_ms_per_pack_max": float(np.max(host_ms[1:])), "host_first_pack_ms": host_ms[0],
+          "k11_ms_per_step": t, "k11_ms_min": float(np.min(steady)),
+          "k11_first_step_ms": ms[0], "planes_per_step": new_planes[1], "planes_first_step": new_planes[0],
+          "algorithmic_bytes_per_step": algo, "GBps": algo / t / 1e6, "frac": algo / t / 1e6 / peak,
+          "peak_GBps": peak, "peak_source": peak_kind, "l2": "256 MB overwritten before every step",
+          "h2d_bytes_per_step": stack_bytes,
+          "what": "host: wall time of DeviceFrameStackPacker.pack on a NumPy step; K11: CUDA events "
+                  "around the three launches of one step"}
+
+
+def collect_arm(nenvs, horizon, rollouts, device):
+  import derl_b200 as d
+
+  def runner(**kw):
+    env = BankEnv(nenvs, seed=4)
+    return d.EnvRunner(env, SyncPolicy(nenvs, device), horizon, nsteps=10 ** 12, **kw).run()
+
+  def timed(it):
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    out = next(it)
+    torch.cuda.synchronize()
+    return time.perf_counter() - t0, out
+
+  arms = {"stacked": runner(resident_device=device),
+          "device_packing": runner(resident_device=device, pack_frames=True)}
+  sec = {name: [] for name in arms}
+  planes = None
+  for i in range(rollouts + 1):
+    for name, it in arms.items():
+      s, out = timed(it)
+      if name == "device_packing":
+        planes = out["observations"].num_frames
+      del out
+      if i:
+        sec[name].append(s)
+  del arms
+  torch.cuda.empty_cache()
+  env, policy = BankEnv(nenvs, seed=4), SyncPolicy(nenvs, device)
+  obs = env.reset()
+  t0 = time.perf_counter()
+  for _ in range(horizon):
+    policy.act(obs)
+    obs = env.step(None)[0]
+  env_s = time.perf_counter() - t0
+  host_s, out = timed(runner(pack_frames=True))
+  host_planes = out["observations"].num_frames
+  del out
+  result = {"envs": nenvs, "horizon": horizon, "rollouts": rollouts,
+            "env_and_policy_s": env_s, "host_packing_s": host_s, "host_packing_planes": host_planes,
+            "device_packing_planes": planes,
+            "what": "seconds per rollout of EnvRunner.run (resident_device unless host_packing), "
+                    "a bank-fed stacking env and a policy that reads its output back each step; "
+                    "host_packing is one first rollout (its pinned plane store is allocated in it)"}
+  for name, s in sec.items():
+    result[name + "_s"] = float(np.mean(s))
+    result[name + "_s_each"] = [float(x) for x in s]
+  return result
 
 
 def kernel_arm(stacked_obs, packed_obs, reps, mb_rows, peak, peak_kind):
@@ -155,6 +311,10 @@ def main():
   p.add_argument("--kernel-reps", type=int, default=40)
   p.add_argument("--steps", type=int, default=3, help="timed updates per arm (update, e2e)")
   p.add_argument("--packer-only", action="store_true")
+  p.add_argument("--pack-only", action="store_true",
+                 help="packer, device_packer and collect arms only")
+  p.add_argument("--pack-steps", type=int, default=64, help="steps timed by device_packer")
+  p.add_argument("--collect-rollouts", type=int, default=2)
   p.add_argument("--no-capacity", action="store_true")
   p.add_argument("--no-e2e", action="store_true")
   cli = p.parse_args()
@@ -176,6 +336,14 @@ def main():
   samples = horizon * nenvs * args.epochs
   peak, peak_kind = bench.peaks()
   line["gpu"] = gpu_info(0)
+  line["device_packer"] = device_packer_arm(cli.envs, cli.pack_steps, peak, peak_kind, device)
+  torch.cuda.empty_cache()
+  line["collect"] = collect_arm(cli.envs, cli.horizon, cli.collect_rollouts, device)
+  torch.cuda.empty_cache()
+  if cli.pack_only:
+    line["gpu_after"] = gpu_info(0)
+    print(json.dumps(line), flush=True)
+    return
 
   stacked, packed = d.make_frame_stack_rollout(horizon, nenvs, device=device, seed=1000)
   line["rollout"] = {"envs": nenvs, "horizon": horizon,
